@@ -11,6 +11,7 @@ emits its consolidated row block of C; no collective follows the multiply (stron
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU code (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's C to DIR/*.npy
 
 At N=1 the JSON line also carries, under "also", BASELINE config 2 (consolidate of a 200M-entry
 COO) and config 3 (regridding SpGEMM), each with its own roofline fraction, and the CPU baseline.
@@ -340,14 +341,18 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         acc = []
         e0.record(stream)
-        for _ in range(args.steps):
+        for k in range(args.steps):
             Cm, sts = hot_path(A_raw, B_raw, w)
             acc.append(sts)
-            Cm.free()
+            if k < args.steps - 1 or not args.dump_outputs:
+                Cm.free()
         e1.record(stream)
         barrier()
         clocks = sampler.stop() if sampler else None
         l1 = launches()
+        if args.dump_outputs:
+            dump_result(torch, Cm, args.dump_outputs, rank, world)
+            Cm.free()
         # partition-independent fingerprints of C (one extra, untimed step): exact wrap-around checksum of the
         # index structure and the fp64 sum of the values -- equal at every N if the row blocks tile C correctly
         Cm, _ = hot_path(A_raw, B_raw, w)
@@ -609,6 +614,33 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ENTRIES = 1 << 21   # 3 arrays x 8 B x 2^21 entries = 48 MB over all ranks, under the 64 MB a dump may take
+DUMP_SEED = 0x5EED00D0
+
+
+def dump_result(torch, Cm, out_dir, rank, world):
+    """--dump-outputs: the C of the timed path's last step, as a caller receives it, written as <out_dir>/C_row.npy,
+    C_col.npy and C_val.npy in float64 (int32 indices are exact in it).  At N > 1 every rank writes its own row block,
+    with a .rank<r> suffix, and takes an equal share of the DUMP_ENTRIES entries.  A block larger than its share is
+    sampled at positions drawn with a fixed seed, in order: the same positions for the same nnz, so two builds can be
+    compared entry for entry."""
+    os.makedirs(out_dir, exist_ok=True)
+    nc = Cm.size()
+    share = DUMP_ENTRIES // world
+    (c0, c1), cv = Cm.device_ptrs()
+    pos = None
+    if nc > share:
+        pos = torch.as_tensor(np.sort(np.random.default_rng(DUMP_SEED).choice(nc, share, replace=False)), device="cuda")
+    suffix = f".rank{rank}" if world > 1 else ""
+    for name, ptr, typestr in (("C_row", c0, "<i4"), ("C_col", c1, "<i4"), ("C_val", cv, "<f8")):
+        if nc == 0:
+            a = np.empty(0, np.float64)
+        else:
+            t = torch.as_tensor(DevView(ptr, nc, typestr), device="cuda")
+            a = (t if pos is None else t[pos]).to(torch.float64).cpu().numpy()
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def e2e_other_apis(ctx, sp, torch, args, m, hA, hB, w_host, nA, nB, fingerprint):
     """The same step end to end through the entry points a user of the reference binds, with PAGEABLE host memory (what
     std::vector is), beside the pinned + pre-wrapped pipeline above:
@@ -643,7 +675,7 @@ def e2e_other_apis(ctx, sp, torch, args, m, hA, hB, w_host, nA, nB, fingerprint)
         del idx, val
     out["cabi_pageable"] = {"ms_per_step": float(np.mean(ms)), "value": 25.0 * m / (float(np.mean(ms)) * 1e-3), "unit": UNIT,
                             "h2d_bytes_per_step": 16.0 * nA + 16.0 * nB + 12.0 * m, "d2h_bytes_per_step": 16.0 * F["nnz_c"],
-                            "result_matches_device_run": bool(ok),
+                            "result_matches_device_run": bool(ok), "steps": len(ms),
                             "api": "pageable numpy arrays -> spb_coo_upload x3 -> spb_multiply_mm (consolidates A and B itself) -> spb_coo_download; one step at a time"}
     del a, b
     return out
@@ -667,6 +699,7 @@ def e2e_cpp_api(ctx, torch, args, m, fingerprint):
             out["cpp_api"] = {"ms_per_step": j["ms_per_step"], "ms_best": j["ms_best"], "value": 25.0 * m / (j["ms_per_step"] * 1e-3), "unit": UNIT,
                               "h2d_bytes_per_step": j["h2d_bytes_per_step"], "d2h_bytes_per_step": j["d2h_bytes_per_step"],
                               "result_matches_device_run": (j["index_checksum"] - F["index_checksum"]) % (1 << 64) == 0 and j["nnz_c"] == F["nnz_c"],
+                              "steps": min(args.steps, 2),
                               "api": "spsparse::multiply(C, 1.0, NULL, A, '.', &w, B, '.', NULL) on VectorCooArray<int,double,2> (std::vector storage), include/spsparse/; tools/cpp/e2e_multiply.cpp"}
         except Exception as e:  # noqa: BLE001 -- a missing leg is reported, not fatal
             out["cpp_api"] = {"unavailable": repr(e)[:300]}
@@ -984,7 +1017,10 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline, of the pinned end-to-end pipeline and of "
+                                                       "'also' configs 2, 3 and 4 (one call); the pageable C-ABI and C++-API end-to-end legs "
+                                                       "(seconds per step) time min(steps, 2), reported as their own 'steps', and config 4 "
+                                                       "as named times one sweep of its row panels")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=100_000_000, help="rows of the banded problem (headline: 1e8)")
@@ -1003,7 +1039,11 @@ def main():
     ap.add_argument("--no-also", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-only", action="store_true", help="only the CPU baselines (with --cpu-full: BASELINE.md section 5's full sizes), no GPU work")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/*.npy (float64, at most 64 MB: "
+                                                          "a fixed, seeded sample of a larger result)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         print(f"note: warmup {args.warmup} < 3 breaks the timing rules", file=sys.stderr)
     if args.impl == "reference":

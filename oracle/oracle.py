@@ -291,10 +291,22 @@ class Impl:
         return sec, n_out.value, s.value
 
 
+def reference_dir():
+    """The checkout of the original spsparse (github.com/citibeth/spsparse) that SPSPARSE_REFERENCE names, or None when
+    the variable is unset.  A value that names no such checkout is an error, not a reason to skip the reference."""
+    d = os.environ.get("SPSPARSE_REFERENCE")
+    if not d:
+        return None
+    if not (os.path.isfile(os.path.join(d, "slib", "spsparse", "spsparse.cpp")) and os.path.isdir(os.path.join(d, "tests"))):
+        raise FileNotFoundError(f"SPSPARSE_REFERENCE={d!r} is not a checkout of spsparse (slib/spsparse/spsparse.cpp and tests/)")
+    return d
+
+
 def build(ref: bool = True) -> None:
-    """Compile the oracle (and, when /root/reference is present, the genuine reference)."""
+    """Compile the oracle (and, when SPSPARSE_REFERENCE names a checkout of the original spsparse, the genuine
+    reference; oracle/Makefile reads the same variable)."""
     subprocess.run(["make", "-s", "-C", HERE, "oracle"], check=True)
-    if ref and os.path.isdir("/root/reference/slib"):
+    if ref and reference_dir():
         subprocess.run(["make", "-s", "-C", HERE, "ref"], check=True)
 
 

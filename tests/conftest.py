@@ -16,12 +16,3 @@ def pytest_configure(config):
 def orc():
     from oracle import oracle as O
     return O.port()
-
-
-@pytest.fixture(scope="session")
-def ref():
-    from oracle import oracle as O
-    r = O.reference()
-    if r is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return r

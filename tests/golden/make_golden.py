@@ -1,9 +1,13 @@
 """Regenerates tests/golden/*.npz from the GENUINE reference (oracle/_ref/libspsparse_ref.so).
 
-Run in the dev container only (needs /root/reference to build oracle/_ref):
-    make -C oracle ref && python tests/golden/make_golden.py
+Needs a checkout of the original spsparse to build oracle/_ref:
+    SPSPARSE_REFERENCE=<checkout> make -C oracle ref && python tests/golden/make_golden.py
 The fixtures pin the oracle (tests/test_oracle_golden.py) and the CUDA path (tests/test_gpu_*.py)
-to the reference's own outputs; they travel to the GPU box, /root/reference does not.
+to the reference's own outputs, so the tests need no copy of the reference.  Packs over 1 MB are stored in parts
+(tests/golden/_pack.py).
+
+    python tests/golden/make_golden.py live               # live_cases: the reference's answers for tests/test_oracle_vs_reference.py
+    python tests/golden/make_golden.py live restatement   # ... written from the restatement instead (see live_cases)
 """
 import ctypes as C
 import os
@@ -21,7 +25,6 @@ from _pack import Packer  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ref = O.reference()
-assert ref is not None, "build oracle/_ref first"
 
 
 def put(d, prefix, coo):
@@ -68,6 +71,52 @@ def dense_ops():
         put(d, f"d{s}_sparse", ref.to_sparse(dense))
     d["count"] = np.array(nd)
     d.save(os.path.join(HERE, "dense_ops_cases.npz"))
+
+
+def live_cases(impl):
+    """The answers tests/test_oracle_vs_reference.py compares the restatement with, on its own seeded inputs (the same
+    loops as there).  The committed live_cases pack was written by `live restatement`: the restatement's answers,
+    which that test, run live against the genuine reference, found identical on every one of these inputs (commit
+    5e24c53, whose CPU suite passed in full with oracle/_ref built; spsparse_oracle.c, _cases.py and the test are
+    unchanged since).  `live` rewrites the pack from the reference itself."""
+    orc = O.port()
+    d = Packer()
+    for s in range(120, 260):
+        c = _cases.consolidate_case(s)
+        a = O.Coo(tuple(c["shape"]), c["idx"], c["val"])
+        r = impl.consolidate(a, tuple(c["sort_order"]), c["policy"], c["zero_nan"])
+        put(d, f"c{s}_out", r)
+        d[f"c{s}_perm"] = impl.sorted_permutation(a, tuple(c["sort_order"]))
+        if a.rank == 2:
+            d[f"c{s}_db"] = impl.dim_beginnings(r)
+    for s in range(300, 700):
+        c = _cases.mm_case(s, big=(s % 40 == 0))
+        A, B = c["A"], c["B"]
+        acon = orc.consolidate(A, (1, 0) if c["tA"] == "T" else (0, 1), c["policy"], c["zero_nan"])
+        bcon = orc.consolidate(B, (0, 1) if c["tB"] == "T" else (1, 0), c["policy"], c["zero_nan"])
+        if (A.n and not acon.n) or (B.n and not bcon.n):
+            continue  # the reference segfaults here (see main)
+        put(d, f"m{s}_out", impl.multiply_mm(c["C"], c["si"], A, c["tA"], c["sj"], B, c["tB"], c["sk"], c["policy"], c["zero_nan"]))
+    for s in range(150, 400):
+        c = _cases.mv_case(s)
+        acon = orc.consolidate(c["A"], (1, 0) if c["tA"] == "T" else (0, 1), c["policy"], c["zero_nan"])
+        if c["A"].n and not acon.n:
+            continue  # reference UB: empty consolidated A
+        put(d, f"v{s}_out", impl.multiply_mv(c["C"], c["si"], c["A"], c["tA"], c["sj"], c["V"], c["policy"], c["zero_nan"]))
+    rng = np.random.default_rng(7)
+    for i in range(300):
+        lists = [np.unique(rng.integers(0, 30, int(rng.integers(0, 20)))).astype(np.int32) for _ in range(3)]
+        d[f"j{i}_2"] = impl.join(lists[0], lists[1])
+        d[f"j{i}_3"] = impl.join(*lists)
+    for s in range(100, 220):
+        c = _cases.dense_case(s)
+        a = O.Coo(tuple(c["shape"]), c["idx"], c["val"])
+        put(d, f"d{s}_T", impl.transpose(a, tuple(c["perm"])))
+        for policy in _cases.POLICIES:
+            dense = impl.to_dense(a, policy)
+            d[f"d{s}_dense{policy}"] = dense
+        put(d, f"d{s}_sparse", impl.to_sparse(dense))
+    return d.save(os.path.join(HERE, "live_cases.npz"))
 
 
 def main():
@@ -152,7 +201,13 @@ def main():
 
 
 if __name__ == "__main__":
-    if sys.argv[1:] == ["dense"]:  # only the newest pack
+    if sys.argv[1:] == ["live", "restatement"]:
+        print(live_cases(O.port()))
+        sys.exit()
+    assert ref is not None, "build oracle/_ref first"
+    if sys.argv[1:] == ["live"]:
+        print(live_cases(ref))
+    elif sys.argv[1:] == ["dense"]:  # only the newest pack
         dense_ops()
     else:
         main()

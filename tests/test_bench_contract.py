@@ -102,3 +102,53 @@ def test_numa_binding_reads_sysfs_and_never_fails(monkeypatch):
     assert bench.bind_to_gpu_numa_node(torch, 0)["bound"] is False
     monkeypatch.setenv("SPB_NO_NUMA_BIND", "1")
     assert bench.bind_to_gpu_numa_node(torch, 0) == {"bound": False, "why": "SPB_NO_NUMA_BIND"}
+
+
+def test_dump_outputs_writes_c_whole_or_as_a_fixed_sample(monkeypatch, tmp_path):
+    """--dump-outputs: C's rows, columns and values as float64 .npy files; a small C whole, a large one at seeded
+    positions in order -- the same positions in every run, and the same for all three arrays -- under 64 MB in all, at
+    N = 1 and over the ranks of N = 8.  Host arrays stand in for the device memory of the result; every value encodes its
+    row and column, so entries taken from different positions cannot pass."""
+    import numpy as np
+    import torch
+    bench = _bench()
+    rng = np.random.default_rng(3)
+    n = bench.DUMP_ENTRIES + 1000
+    row = np.sort(rng.integers(0, 1 << 20, n)).astype(np.int32)
+    col = rng.integers(0, 1 << 20, n).astype(np.int32)
+    arrays = [row, col, row * float(1 << 20) + col]
+
+    class Result:
+        def __init__(self, size):
+            self.n = size
+
+        def size(self):
+            return self.n
+
+        def device_ptrs(self):
+            return (0, 1), 2
+
+    def as_tensor(x, device=None):
+        if isinstance(x, bench.DevView):
+            iface = x.__cuda_array_interface__
+            return torch.from_numpy(arrays[iface["data"][0]][:iface["shape"][0]])
+        return torch.from_numpy(np.asarray(x))
+    monkeypatch.setattr(torch, "as_tensor", as_tensor)
+    for size, d in ((1000, "small"), (n, "a"), (n, "b")):
+        bench.dump_result(torch, Result(size), str(tmp_path / d), 0, 1)
+    names = ("C_row.npy", "C_col.npy", "C_val.npy")
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(names)
+    for name, a in zip(names, arrays):
+        small = np.load(tmp_path / "small" / name)
+        assert small.dtype == np.float64 and np.array_equal(small, a[:1000])
+        x, y = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert x.dtype == np.float64 and len(x) == bench.DUMP_ENTRIES and x.tobytes() == y.tobytes()
+    r, c, v = (np.load(tmp_path / "a" / name) for name in names)
+    assert np.array_equal(v, r * (1 << 20) + c) and np.isin(v, arrays[2]).all()    # whole entries of C
+    assert np.all(np.diff(r) >= 0)                                                   # positions in order: rows stay sorted
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in names) <= 64 << 20
+    for rank in range(8):                                                            # N = 8: every rank its own block
+        bench.dump_result(torch, Result(n), str(tmp_path / "n8"), rank, 8)
+    files = os.listdir(tmp_path / "n8")
+    assert sorted(files) == sorted(f"{name[:-4]}.rank{rank}.npy" for name in names for rank in range(8))
+    assert sum(os.path.getsize(tmp_path / "n8" / f) for f in files) <= 64 << 20

@@ -2,8 +2,8 @@
 
 (1) tests/cpp/host_layer_test.cpp: this repo's own C++ test of the template API.
 (2) the REFERENCE's own gtest sources (tests/test_xiter.cpp, test_array.cpp, test_multiply_sparse.cpp),
-    compiled UNMODIFIED against this repo's headers by `make -C oracle dropin` in the dev container
-    (the sources stay in /root/reference; only the binaries travel, under oracle/_ref/).
+    compiled UNMODIFIED against this repo's headers by `make -C oracle dropin` when SPSPARSE_REFERENCE names a
+    checkout of the original spsparse (the sources stay there; the binaries go to oracle/_ref/).
 """
 import os
 import subprocess
@@ -31,6 +31,6 @@ def test_host_layer_cpp():
 def test_reference_sources_against_our_headers(name):
     exe = os.path.join(ROOT, "oracle", "_ref", "dropin_" + name)
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/dropin_* not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/dropin_* not built (needs SPSPARSE_REFERENCE, a checkout of the original spsparse, at build time)")
     rc, out = run(exe)
     assert rc == 0 and " 0 failed" in out, out

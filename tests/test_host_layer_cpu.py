@@ -3,7 +3,7 @@
 (1) tests/cpp/host_only_test.cpp -- container, accessors, iterators, sorted joins, accumulators, error hook and the
     short-circuits of consolidate/multiply that return before any device work (SURVEY 8a rows a1, a2, a6, a8, a12).
 (2) the REFERENCE's own tests/test_xiter.cpp, compiled unmodified against this repo's headers (oracle/_ref/dropin_test_xiter,
-    built by `make -C oracle dropin` where /root/reference exists): joins are pure host code, so it runs without a GPU.
+    built by `make -C oracle dropin` when SPSPARSE_REFERENCE names a checkout of it): joins are pure host code, so it runs without a GPU.
 Everything that computes on the device is in test_gpu_dropin.py.
 """
 import os
@@ -24,6 +24,6 @@ def test_host_only_cpp():
 def test_reference_xiter_source_against_our_headers():
     exe = os.path.join(ROOT, "oracle", "_ref", "dropin_test_xiter")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/dropin_test_xiter not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/dropin_test_xiter not built (needs SPSPARSE_REFERENCE, a checkout of the original spsparse, at build time)")
     r = subprocess.run([exe], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and " 0 failed" in r.stdout, r.stdout[-4000:] + r.stderr[-2000:]

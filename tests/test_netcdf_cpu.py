@@ -213,6 +213,6 @@ def test_single_record_variable_is_not_padded(exe, tmp_path):
 def test_reference_netcdf_test_against_our_headers(tmp_path):
     exe = os.path.join(ROOT, "oracle", "_ref", "dropin_test_netcdf")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/dropin_test_netcdf not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/dropin_test_netcdf not built (needs SPSPARSE_REFERENCE, a checkout of the original spsparse, at build time)")
     r = subprocess.run([exe], capture_output=True, text=True, timeout=120, cwd=str(tmp_path))
     assert r.returncode == 0 and " 0 failed" in r.stdout, r.stdout[-4000:] + r.stderr[-2000:]
