@@ -82,14 +82,32 @@ __global__ void k_scatter_row_len(const u32 *__restrict__ row_start, const i32 *
 // Dense pointer straight from the compressed rows: ptr[v] = offset of the first entry whose leading index is >= v, for v in
 // [0, extent].  Compressed row t fills the values (id[t-1], id[t]] -- the empty rows in front of it and itself -- and the last
 // one also everything behind it.  One read of the compressed rows, one write of the pointer; no zero-fill, no scan.
-__global__ void k_dense_ptr_from_rows(const u32 *__restrict__ row_start, const i32 *__restrict__ row_id, u32 nrows, u32 n, u64 extent, u32 *ptr) {
+// A stretch longer than DP_LONG_GAP values (rows {0, 2^31-1}: one thread would write 2^31 words) is not written by its
+// thread but appended to `gaps`, and k_fill_gaps writes it with the whole grid.  Such a stretch needs at least DP_LONG_GAP
+// empty rows, so the caller passes gaps = nullptr when extent + 1 - nrows is smaller: every thread then writes its own.
+constexpr u64 DP_LONG_GAP = 4096;
+struct DpGap { u64 lo, end; u32 value; };
+__device__ __forceinline__ void dp_fill(u32 *ptr, u64 lo, u64 end, u32 value, DpGap *gaps, u32 *n_gaps) {
+    if (gaps && end - lo > DP_LONG_GAP) {
+        gaps[atomicAdd(n_gaps, 1u)] = DpGap{lo, end, value};
+        return;
+    }
+    for (u64 v = lo; v < end; ++v) ptr[v] = value;
+}
+__global__ void k_dense_ptr_from_rows(const u32 *__restrict__ row_start, const i32 *__restrict__ row_id, u32 nrows, u32 n, u64 extent, u32 *ptr,
+                                      DpGap *gaps, u32 *n_gaps) {
     for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < nrows; t += (u64)gridDim.x * blockDim.x) {
         const u64 hi = (u64)(u32)row_id[t];
         const u64 lo = t ? (u64)(u32)row_id[t - 1] + 1 : 0;
-        const u32 at = row_start[t];
-        for (u64 v = lo; v <= hi; ++v) ptr[v] = at;
-        if (t + 1 == nrows)
-            for (u64 v = hi + 1; v <= extent; ++v) ptr[v] = n;
+        dp_fill(ptr, lo, hi + 1, row_start[t], gaps, n_gaps);
+        if (t + 1 == nrows) dp_fill(ptr, hi + 1, extent + 1, n, gaps, n_gaps);
+    }
+}
+__global__ void k_fill_gaps(const DpGap *__restrict__ gaps, const u32 *n_gaps, u32 *ptr) {
+    const u32 ng = *n_gaps;
+    for (u32 g = 0; g < ng; ++g) {
+        const DpGap d = gaps[g];
+        for (u64 v = d.lo + (u64)blockIdx.x * blockDim.x + threadIdx.x; v < d.end; v += (u64)gridDim.x * blockDim.x) ptr[v] = d.value;
     }
 }
 __global__ void k_fill_u32(u32 *p, u64 count, u32 value) {

@@ -1019,9 +1019,17 @@ static int build_dense_ptr(spb_ctx *ctx, const spb_coo *a_const, u64 extent, u32
         CKR(build_row_index(ctx, a, &ri));
         CK(ctx->pool.alloc((void **)&a->dense_ptr, (extent + 2) * sizeof(u32)));
         // straight from the compressed rows (one read, one write; nothing is read back: no host synchronisation)
+        Scratch ws(ctx);
+        DpGap *gaps = nullptr;
+        u32 *n_gaps = nullptr;
+        if (ri.nrows && extent + 1 - ri.nrows >= DP_LONG_GAP) {   // long stretches of empty rows are possible: list them
+            CKR(ws.get(&gaps, (extent + 1) / DP_LONG_GAP + 1));
+            CKR(ws.zeroed(&n_gaps, 1));
+        }
         ++ctx->launches;
-        if (ri.nrows) k_dense_ptr_from_rows<<<grid_for(ri.nrows, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(ri.start, ri.id, ri.nrows, (u32)a->n, extent, a->dense_ptr);
+        if (ri.nrows) k_dense_ptr_from_rows<<<grid_for(ri.nrows, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(ri.start, ri.id, ri.nrows, (u32)a->n, extent, a->dense_ptr, gaps, n_gaps);
         else k_fill_u32<<<grid_for(extent + 1, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(a->dense_ptr, extent + 1, 0u);
+        if (gaps) ++ctx->launches, k_fill_gaps<<<(u32)ctx->sm_count * 8, 256, 0, ctx->stream>>>(gaps, n_gaps, a->dense_ptr);
         CK(cudaGetLastError());
     }
     *ptr_out = a->dense_ptr;

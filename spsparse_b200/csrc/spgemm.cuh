@@ -63,7 +63,7 @@ __global__ void k_row_maxlen(const u32 *__restrict__ row_start, u32 nrows, u32 *
 __global__ void k_entry_products(MMOperands m, const i32 *__restrict__ a_row, u32 *ent_f) {
     for (u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x; e < m.nnz_a; e += (u64)gridDim.x * blockDim.x) {
         i32 j = m.a_j[e];
-        u32 f = m.bptr[j + 1] - m.bptr[j];
+        u32 f = m.bptr[(u32)j + 1] - m.bptr[j];
         if (m.sj_mask && !m.sj_mask[j]) f = 0;
         if (m.si && m.si[a_row[e]] == 0.0) f = 0;
         ent_f[e] = f;
@@ -109,6 +109,9 @@ __global__ void k_esc_row_products(MMOperands m, const u64 *__restrict__ ent_off
 // ---- short rows: k-way merge in registers, one thread per row -----------------------------------
 // The heads of up to NL column-sorted B rows live in registers; each step takes the smallest head
 // column, sums every list that holds it in list (= ascending j) order and advances those lists.
+// Heads are compared unsigned and an exhausted list holds MERGE_END, a value no column can take (columns are < 2^31):
+// column 2^31-1 = INT32_MAX is a real column of a matrix 2^31 wide.
+constexpr u32 MERGE_END = 0xffffffffu;
 // Where a merge reads B from: the global arrays (k0 = j0 = 0, read-only cache loads), or -- LOCAL -- the copies a block made in
 // shared memory of the stretch of B its rows reference (k0 / j0 = first entry / first row of that stretch).
 struct BView {
@@ -124,7 +127,7 @@ template <bool LOCAL> __device__ __forceinline__ u32 bv_p(const BView &b, u32 j)
 template <int NL, bool LOCAL = false>
 struct RowMerge {
     u32 cur[NL], end[NL];
-    i32 hk[NL];
+    u32 hk[NL];   // head column, MERGE_END once the list is exhausted
     double hv[NL], as[NL];
     BView b;
 
@@ -134,7 +137,7 @@ struct RowMerge {
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
             cur[l] = end[l] = 0;
-            hk[l] = INT32_MAX;
+            hk[l] = MERGE_END;
             hv[l] = 0.0;
             as[l] = 0.0;
             if ((u32)l < len) {
@@ -146,7 +149,7 @@ struct RowMerge {
                     end[l] = bv_p<LOCAL>(b, (u32)j + 1);
                     as[l] = m.sj ? __dmul_rn(a, __ldg(m.sj + j)) : a;  // (a*s) first, multiply_sparse.hpp:228
                     if (cur[l] < end[l]) {
-                        hk[l] = bv_k<LOCAL>(b, cur[l]);
+                        hk[l] = (u32)bv_k<LOCAL>(b, cur[l]);
                         hv[l] = bv_v<LOCAL>(b, cur[l]);
                     }
                 }
@@ -168,10 +171,10 @@ struct RowMerge {
 
     // Next output column and its dot product; false when every list is exhausted.
     __device__ __forceinline__ bool next(const MMOperands &m, i32 &k, double &sum) {
-        i32 kmin = hk[0];
+        u32 kmin = hk[0];
 #pragma unroll
         for (int l = 1; l < NL; ++l) kmin = min(kmin, hk[l]);
-        if (kmin == INT32_MAX) return false;
+        if (kmin == MERGE_END) return false;
         double acc = 0.0;  // multiply_sparse.hpp:219
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
@@ -179,14 +182,14 @@ struct RowMerge {
                 acc = __dadd_rn(acc, __dmul_rn(as[l], hv[l]));
                 ++cur[l];
                 if (cur[l] < end[l]) {
-                    hk[l] = bv_k<LOCAL>(b, cur[l]);
+                    hk[l] = (u32)bv_k<LOCAL>(b, cur[l]);
                     hv[l] = bv_v<LOCAL>(b, cur[l]);
                 } else {
-                    hk[l] = INT32_MAX;
+                    hk[l] = MERGE_END;
                 }
             }
         }
-        k = kmin;
+        k = (i32)kmin;
         sum = acc;
         return true;
     }
@@ -200,7 +203,7 @@ struct RowMerge {
 template <int NL, bool LOCAL = false>
 struct RowMergeK {
     u32 cur[NL], end[NL];
-    i32 hk[NL];
+    u32 hk[NL];   // as in RowMerge
     BView b;
     __device__ __forceinline__ void init(const MMOperands &m, u32 s, u32 len, const BView *view = nullptr) {
         if (view) b = *view;
@@ -208,30 +211,30 @@ struct RowMergeK {
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
             cur[l] = end[l] = 0;
-            hk[l] = INT32_MAX;
+            hk[l] = MERGE_END;
             if ((u32)l < len) {
                 const i32 j = __ldg(m.a_j + s + l);
                 if (!m.sj_mask || m.sj_mask[j]) {
                     cur[l] = bv_p<LOCAL>(b, (u32)j);
                     end[l] = bv_p<LOCAL>(b, (u32)j + 1);
-                    if (cur[l] < end[l]) hk[l] = bv_k<LOCAL>(b, cur[l]);
+                    if (cur[l] < end[l]) hk[l] = (u32)bv_k<LOCAL>(b, cur[l]);
                 }
             }
         }
     }
     __device__ __forceinline__ bool next(i32 &k) {
-        i32 kmin = hk[0];
+        u32 kmin = hk[0];
 #pragma unroll
         for (int l = 1; l < NL; ++l) kmin = min(kmin, hk[l]);
-        if (kmin == INT32_MAX) return false;
+        if (kmin == MERGE_END) return false;
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
             if (hk[l] == kmin) {
                 ++cur[l];
-                hk[l] = cur[l] < end[l] ? bv_k<LOCAL>(b, cur[l]) : INT32_MAX;
+                hk[l] = cur[l] < end[l] ? (u32)bv_k<LOCAL>(b, cur[l]) : MERGE_END;
             }
         }
-        k = kmin;
+        k = (i32)kmin;
         return true;
     }
 };
@@ -742,7 +745,7 @@ __global__ void __launch_bounds__(128) k_hash_win_bounds(MMOperands m, HashArgs 
             const u32 x = t / nb, w = t % nb + 1;
             const i32 j = m.a_j[s + x];
             const u64 col = (u64)w * a.win_cols;
-            const u32 bs = m.bptr[j], be = m.bptr[j + 1];
+            const u32 bs = m.bptr[j], be = m.bptr[(u32)j + 1];
             win_bound[(u64)(s + x) * nb + (w - 1)] = col <= (u64)INT32_MAX ? hn_lower_bound(m.b_k, bs, be, (i32)col) : be;
         }
     }
@@ -837,7 +840,7 @@ __global__ void __launch_bounds__(HS_THREADS, 1) k_hash_symbolic(MMOperands m, H
                 const i32 j = m.a_j[ent];
                 if (!m.sj_mask || m.sj_mask[j]) {
                     bs = m.bptr[j];
-                    u32 be = m.bptr[j + 1];
+                    u32 be = m.bptr[(u32)j + 1];
                     if (a.n_win > 1 && a.win_bound) {
                         const u32 *wb = a.win_bound + (u64)ent * (a.n_win - 1);
                         if (win > 0) bs = wb[win - 1];
@@ -1090,7 +1093,7 @@ __global__ void __launch_bounds__(HSM_THREADS) k_hash_symbolic_small(MMOperands 
             u32 bs = 0, len = 0;
             if (ent < e) {
                 const i32 j = m.a_j[ent];
-                if (!m.sj_mask || m.sj_mask[j]) { bs = m.bptr[j]; len = m.bptr[j + 1] - bs; }
+                if (!m.sj_mask || m.sj_mask[j]) { bs = m.bptr[j]; len = m.bptr[(u32)j + 1] - bs; }
             }
             u32 nE, Tc;
             __syncthreads();   // the previous chunk's staging (and the previous row's keys) are no longer read
@@ -1189,7 +1192,7 @@ __global__ void __launch_bounds__(256) k_hash_splits(MMOperands m, HashArgs a, u
         u32 *dst = split + a.row_split[sr] + (u64)(part - 1) * len;
         for (u32 x = threadIdx.x; x < len; x += blockDim.x) {
             const i32 j = m.a_j[s + x];
-            dst[x] = hn_lower_bound(m.b_k, m.bptr[j], m.bptr[j + 1], key);
+            dst[x] = hn_lower_bound(m.b_k, m.bptr[j], m.bptr[(u32)j + 1], key);
         }
     }
 }
@@ -1291,7 +1294,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) k_hash_numeric(MMOperands m, Ha
                 if (split_hi) w_hi = split_hi[ent - s];
                 if (!m.sj_mask || m.sj_mask[j]) {
                     bs = split_lo ? w_lo : m.bptr[j];
-                    const u32 be = split_hi ? w_hi : m.bptr[j + 1];
+                    const u32 be = split_hi ? w_hi : m.bptr[(u32)j + 1];
                     len = be - bs;
                     as = m.a_val[ent];
                     if (m.sj) as = __dmul_rn(as, m.sj[j]);  // (a*s) first, :228
