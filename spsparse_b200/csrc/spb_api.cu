@@ -60,6 +60,10 @@ struct DevPool {
     std::unordered_map<void *, size_t> live_;
     std::mutex mu_;
     size_t cached_bytes = 0;
+    // SPB_POOL_POISON (tests): every block handed out is first filled with this byte over its whole size, on `stream`, so a
+    // kernel that reads a slot nobody wrote sees the pattern instead of zeros or the previous call's data; -1 = off
+    int poison = -1;
+    cudaStream_t stream = nullptr;
 
     static size_t round_up(size_t b) {
         if (b < 512) return 512;
@@ -76,8 +80,9 @@ struct DevPool {
             *out = it->second;
             live_[*out] = it->first;
             cached_bytes -= it->first;
+            const size_t got = it->first;
             free_.erase(it);
-            return cudaSuccess;
+            return poison >= 0 ? cudaMemsetAsync(*out, poison, got, stream) : cudaSuccess;
         }
         void *p = nullptr;
         cudaError_t e = cudaMalloc(&p, want);
@@ -89,7 +94,7 @@ struct DevPool {
         }
         live_[p] = want;
         *out = p;
-        return cudaSuccess;
+        return poison >= 0 ? cudaMemsetAsync(p, poison, want, stream) : cudaSuccess;
     }
     void release(void *p) {
         if (!p) return;
@@ -357,7 +362,15 @@ int spb_ctx_create(int device, void *cuda_stream, spb_ctx **out) {
     CK(cudaFuncSetAttribute(k_radix_pass9<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R9_SMEM_BYTES));
     CK(cudaFuncSetAttribute(k_radix_pass9<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R9_SMEM_BYTES));
     c->bulk_load = getenv("SPB_BULK_LOAD") ? atoi(getenv("SPB_BULK_LOAD")) != 0 : true;
-    const char *s = getenv("SPB_MERGE_MAX_PRODUCTS");
+    const char *s = getenv("SPB_POOL_POISON");
+    if (s) {  // one byte in hex: "00", "ff", "7f"
+        char *end = nullptr;
+        const unsigned long b = strtoul(s, &end, 16);
+        if (!*s || *end || b > 0xff) return spb_fail(SPB_ERR_ARG, "SPB_POOL_POISON=%s: expected one byte in hex (00 .. ff)", s);
+        c->pool.poison = (int)b;
+        c->pool.stream = c->stream;
+    }
+    s = getenv("SPB_MERGE_MAX_PRODUCTS");
     c->merge_max_products = s ? (u32)strtoul(s, nullptr, 10) : 1024u;
     s = getenv("SPB_ESC_CHUNK");
     c->esc_chunk = s ? strtoull(s, nullptr, 10) : (1ull << 27);
