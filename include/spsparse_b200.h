@@ -110,6 +110,30 @@ typedef struct {
 int spb_consolidate(spb_ctx *ctx, const spb_coo *in, const int *sort_order, int policy, int zero_nan,
                     spb_coo **out, spb_consolidate_stats *stats /* may be NULL */);
 
+/* ---- consolidate with a fixed index pattern  (spsparse::consolidate, algorithm.hpp:251-319) ----------------------
+ * For callers that assemble the same (row, column) pattern again and again with new values (a time step, a regridding
+ * step): the pattern is sorted once, and every later consolidate of new values over it is one gather pass plus the
+ * duplicate-reduce -- no sort.  The result of a run depends on the values as consolidate's does (zeros dropped, NaNs of the
+ * leading run dropped with zero_nan, the policy's fold) and is bit-identical to spb_consolidate on the same data.
+ *
+ * spb_consolidate_plan_create  sorts the index pattern of `in` once (stable, every entry kept, nothing merged); the values
+ *                              of `in` are not read.  Index bounds are checked here, with spb_consolidate's errors.  `in`
+ *                              may be freed afterwards.  The plan holds 12 bytes of device memory per entry (the sorted
+ *                              packed keys and the 32-bit permutation).  n_runs (may be NULL): distinct index tuples.
+ * spb_consolidate_plan_run     what spb_consolidate(ctx, X, sort_order, policy, zero_nan) returns, where X has the plan's
+ *                              indices and the values `val`: n doubles in the entry order of the array the plan was made
+ *                              from.  `val` may be device memory of the plan's device (any 8-byte alignment) or host memory
+ *                              (staged as spb_coo_upload stages it).  `out` is a new array flagged sorted by sort_order.
+ *                              stats: passes = 0 (no radix pass runs), ms_sort = the gather pass (with zero_nan also the
+ *                              search for the leading run's end), n_kept / n_out of this run.
+ * spb_consolidate_plan_destroy releases the plan; call it before destroying the plan's context. */
+typedef struct spb_cons_plan spb_cons_plan;
+int spb_consolidate_plan_create(spb_ctx *ctx, const spb_coo *in, const int *sort_order, spb_cons_plan **out,
+                                uint64_t *n_runs /* may be NULL */);
+int spb_consolidate_plan_run(spb_cons_plan *plan, const double *val, int policy, int zero_nan, spb_coo **out,
+                             spb_consolidate_stats *stats /* may be NULL */);
+int spb_consolidate_plan_destroy(spb_cons_plan *plan);
+
 /* ---- sorted_permutation  (spsparse::sorted_permutation, algorithm.hpp:411-427) -----------
  * perm[t] = position in `in` of the entry that a stable sort by sort_order puts at position t.
  * Writes in->n values to host memory.  Nothing is dropped or merged. */

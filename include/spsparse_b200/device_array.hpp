@@ -138,6 +138,48 @@ public:
     }
 };
 
+// consolidate for a fixed index pattern (spb_consolidate_plan_*): the pattern of A is sorted once; consolidate(val, ...)
+// returns what A-with-values-val .consolidate(sort_order, ...) would, bit for bit, with one gather pass and the
+// duplicate-reduce instead of a sort.  `val` holds A.size() doubles in A's entry order, in device or host memory.  A may be
+// destroyed once the plan exists.  Move-only; 12 bytes of device memory per entry.
+template <int RANK>
+class ConsolidatePlan {
+    static_assert(RANK == 1 || RANK == 2, "rank 1 and 2 arrays only");
+    spb_cons_plan *h_ = nullptr;
+    size_t n_runs_ = 0;
+
+public:
+    ConsolidatePlan() {}
+    ConsolidatePlan(DeviceCooArray<RANK> const &A, std::array<int, RANK> const &sort_order) {
+        int so[2] = {sort_order[0], RANK > 1 ? sort_order[RANK - 1] : 0};
+        uint64_t runs = 0;
+        check(spb_consolidate_plan_create(default_context(), A.handle(), so, &h_, &runs));
+        n_runs_ = (size_t)runs;
+    }
+    ConsolidatePlan(ConsolidatePlan const &) = delete;
+    ConsolidatePlan &operator=(ConsolidatePlan const &) = delete;
+    ConsolidatePlan(ConsolidatePlan &&o) noexcept : h_(o.h_), n_runs_(o.n_runs_) { o.h_ = nullptr; o.n_runs_ = 0; }
+    ConsolidatePlan &operator=(ConsolidatePlan &&o) noexcept {
+        if (this != &o) { reset(); h_ = o.h_; n_runs_ = o.n_runs_; o.h_ = nullptr; o.n_runs_ = 0; }
+        return *this;
+    }
+    ~ConsolidatePlan() { reset(); }
+    void reset() {
+        if (h_) spb_consolidate_plan_destroy(h_);
+        h_ = nullptr;
+        n_runs_ = 0;
+    }
+    spb_cons_plan *handle() const { return h_; }
+    size_t n_runs() const { return n_runs_; }   // distinct index tuples of the pattern
+
+    DeviceCooArray<RANK> consolidate(const double *val, DuplicatePolicy policy = DuplicatePolicy::ADD,
+                                     bool zero_nan = false) const {
+        spb_coo *r = nullptr;
+        check(spb_consolidate_plan_run(h_, val, policy_code(policy), zero_nan ? 1 : 0, &r, nullptr));
+        return DeviceCooArray<RANK>(r);
+    }
+};
+
 // C * diag(scalei) * op(A) * diag(scalej) * op(B) * diag(scalek); absent scale vectors: nullptr.  Operands need not be
 // consolidated (the library does what the reference's Consolidate<> does); the result is consolidated row-major.
 inline DeviceCooArray<2> multiply(double C, DeviceCooArray<1> const *scalei, DeviceCooArray<2> const &A, char transpose_A,

@@ -72,6 +72,9 @@ SIGNATURES = {
     "spb_coo_free": (C.c_int, [vp, vp]),
     "spb_consolidate": (C.c_int, [vp, vp, intp, C.c_int, C.c_int, C.POINTER(vp), C.POINTER(ConsolidateStats)]),
     "spb_sorted_permutation": (C.c_int, [vp, vp, intp, u64p]),
+    "spb_consolidate_plan_create": (C.c_int, [vp, vp, intp, C.POINTER(vp), u64p]),
+    "spb_consolidate_plan_run": (C.c_int, [vp, vp, C.c_int, C.c_int, C.POINTER(vp), C.POINTER(ConsolidateStats)]),
+    "spb_consolidate_plan_destroy": (C.c_int, [vp]),
     "spb_dim_beginnings": (C.c_int, [vp, vp, u64p, C.c_uint64, u64p]),
     "spb_multiply_mm": (C.c_int, [vp, C.c_double, vp, vp, C.c_char, vp, vp, C.c_char, vp, C.c_int, C.c_int,
                                   C.POINTER(vp), C.POINTER(MMStats)]),

@@ -203,6 +203,49 @@ def consolidate(ctx: Context, A: CooArray, sort_order, duplicate_policy=ADD, zer
     return (out, st) if stats else out
 
 
+class ConsolidatePlan:
+    """``consolidate`` for a fixed index pattern (spb_consolidate_plan_*): the pattern of ``A`` is sorted once, and every
+    ``run(values)`` returns what ``consolidate`` returns for ``A``'s indices with those values -- bit for bit -- with one
+    gather pass and the duplicate-reduce instead of a sort.  ``A`` may be freed once the plan exists.  Device values are read on
+    the context's stream: values written on another stream must be complete (synchronise, or share the stream)."""
+
+    def __init__(self, ctx: Context, A: CooArray, sort_order):
+        self.ctx = ctx
+        self.n = A.size()
+        h, runs = vp(), C.c_uint64()
+        check(ctx.lib.spb_consolidate_plan_create(ctx.h, A.h, _order(sort_order), C.byref(h), C.byref(runs)))
+        self.h, self.n_runs = h, int(runs.value)
+
+    def _values(self, values):
+        """(pointer, keep-alive) for a CUDA float64 tensor, a numpy array (host memory) or a raw device pointer."""
+        if isinstance(values, int):
+            return values, None
+        if isinstance(values, np.ndarray):
+            v = np.ascontiguousarray(values, dtype=np.float64)
+            if v.ndim != 1 or v.shape[0] != self.n:
+                raise ValueError(f"values: {v.shape} for a plan of {self.n} entries")
+            return v.ctypes.data, v
+        if hasattr(values, "data_ptr") and getattr(values, "is_cuda", False):
+            import torch
+            if values.dtype != torch.float64 or values.dim() != 1 or values.numel() != self.n or values.stride(0) != 1:
+                raise ValueError(f"values: need a contiguous float64 tensor of {self.n} entries")
+            return values.data_ptr(), values
+        raise TypeError("values: a CUDA float64 tensor, a numpy array or a device pointer")
+
+    def run(self, values, duplicate_policy=ADD, zero_nan=False, stats=False):
+        ptr, _keep = self._values(values)   # _keep: a converted numpy copy must outlive the call
+        h, st = vp(), ConsolidateStats()
+        check(self.ctx.lib.spb_consolidate_plan_run(self.h, vp(ptr) if ptr else None, int(duplicate_policy),
+                                                    int(bool(zero_nan)), C.byref(h), C.byref(st)))
+        out = CooArray(self.ctx, h)
+        return (out, st) if stats else out
+
+    def free(self):
+        if self.h:
+            self.ctx.lib.spb_consolidate_plan_destroy(self.h)
+            self.h = None
+
+
 def copy(ctx: Context, A: CooArray):
     """spsparse::copy (algorithm.hpp:30-37) into a fresh array."""
     h = vp()

@@ -27,6 +27,7 @@
 #include "spgemm.cuh"
 #include "dense_ops.cuh"
 #include "rowpart.cuh"
+#include "cons_plan.cuh"
 
 thread_local std::string g_last_error;
 
@@ -2037,6 +2038,201 @@ int spb_multiply_mv(spb_ctx *ctx, double C, const spb_coo *si, const spb_coo *A,
     spb_coo_free(ctx, Vc);
     if (rc) { spb_coo_free(ctx, r); *out = nullptr; }
     return rc;
+}
+
+}  // extern "C"
+
+// ---- consolidate with a fixed index pattern ----------------------------------------------------------------------------
+// The pattern is sorted once (cons_plan.cuh); a run gathers the new values into that order, dropping what consolidate()
+// drops, and hands the kept pairs to the duplicate-reduce that sort_reduce runs after its passes.  12 bytes of device memory
+// per entry, from the context's pool.
+struct spb_cons_plan {
+    spb_ctx *ctx;
+    int rank;
+    u64 shape[2];
+    int so[2];
+    u64 n;
+    int bits_lo, key_bits;
+    u64 *keys;   // [n] packed keys (idx[so[0]] << bits_lo) | idx[so[1]], in stable sorted order
+    u32 *perm;   // [n] sorted position -> entry number
+};
+
+// the reduce of the kept pairs into r (allocated for plan->n entries); statistics as spb_consolidate_stats describes
+static int cons_plan_run(spb_cons_plan *plan, const double *dval, int policy, int zero_nan, spb_coo *r,
+                         spb_consolidate_stats *st) {
+    spb_ctx *ctx = plan->ctx;
+    const u32 n = (u32)plan->n;
+    Scratch ws(ctx);
+    Timer tm(ctx->stream);
+    const int t0 = tm.mark();
+    u32 *counters, *tickets, *bound = nullptr;   // counters: [0] kept, [2] out count, [3] long runs, [4] rows
+    u64 *gstate, *kA;
+    double *vA;
+    const u32 tiles = (u32)div_up(n, CP_TILE);
+    CKR(ws.zeroed(&counters, 8));
+    CKR(ws.zeroed(&tickets, 2));
+    CKR(ws.zeroed(&gstate, tiles));
+    CKR(ws.get(&kA, n));
+    CKR(ws.get(&vA, n));
+    if (zero_nan) {
+        CKR(ws.get(&bound, 1));
+        CK(cudaMemsetAsync(bound, 0xFF, sizeof(u32), ctx->stream));
+        const u32 grid = tiles < (u32)ctx->sm_count * 2 ? tiles : (u32)ctx->sm_count * 2;
+        ++ctx->launches, k_plan_first_kept<<<grid, CP_THREADS, 0, ctx->stream>>>(plan->perm, dval, n, tickets + 1, bound);
+    }
+    PlanGatherArgs ga;
+    ga.keys = plan->keys; ga.perm = plan->perm; ga.val = dval; ga.n = n; ga.bound = bound;
+    ga.keys_out = kA; ga.vals_out = vA; ga.n_kept = counters; ga.state = gstate; ga.ticket = tickets;
+    ++ctx->launches, k_plan_gather<<<tiles, CP_THREADS, 0, ctx->stream>>>(ga);
+    CK(cudaGetLastError());
+    const int t1 = tm.mark();
+
+    // the reduce pass sort_reduce runs where no in-row sort counted the heads: a block per tile, placed by a look-back (the
+    // warp-per-tile look-back variant measured slower, DESIGN.md section 3)
+    const u32 rtiles = (u32)div_up(n, RK_TILE);
+    ReduceArgs ra;
+    memset(&ra, 0, sizeof ra);
+    ra.keys = kA; ra.vals = vA; ra.n_ptr = counters; ra.bits_lo = plan->bits_lo; ra.policy = policy;
+    ra.out_hi = r->idx[plan->so[0]]; ra.out_lo = plan->rank > 1 ? r->idx[plan->so[1]] : nullptr; ra.out_val = r->val;
+    ra.out_count = counters + 2;
+    CKR(ws.zeroed(&ra.state, rtiles));
+    CKR(ws.zeroed(&ra.ticket, 1));
+    ra.long_cap = n / RK_LONG_RUN + 1;
+    CKR(ws.get(&ra.long_list, 2ull * ra.long_cap));
+    ra.long_count = counters + 3;
+    ra.row_start = r->row_start; ra.row_id = r->row_id; ra.row_count = counters + 4;
+    ++ctx->launches, k_reduce_by_key<MODE_CONSOLIDATE><<<rtiles, RK_THREADS, 0, ctx->stream>>>(ra);
+    if (policy == POLICY_ADD || policy == POLICY_REPLACE)
+        ++ctx->launches, k_long_runs<<<(u32)ctx->sm_count * 4, 256, 0, ctx->stream>>>(ra);
+    CK(cudaGetLastError());
+    const int t2 = tm.mark();
+
+    u32 h[8];
+    CK(cudaMemcpyAsync(h, counters, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    r->n = h[2];
+    if (plan->rank == 2) {
+        r->nrows = h[4];
+        r->rows_valid = true;
+        if (h[2] == 0) { const u32 z = 0; CK(cudaMemcpyAsync(r->row_start, &z, sizeof z, cudaMemcpyHostToDevice, ctx->stream)); CK(cudaStreamSynchronize(ctx->stream)); }
+    }
+    if (st) {
+        st->n_in = n; st->n_kept = h[0]; st->n_out = h[2];
+        st->key_bits = plan->key_bits; st->passes = 0; st->digit_bits = 0;
+        st->ms_sort = tm.ms(t0, t1); st->ms_reduce = tm.ms(t1, t2); st->ms_total = tm.ms(t0, t2);
+        st->ms_pass = 0.f;
+    }
+    return 0;
+}
+
+extern "C" {
+
+int spb_consolidate_plan_create(spb_ctx *ctx, const spb_coo *in, const int *sort_order, spb_cons_plan **out,
+                                uint64_t *n_runs) {
+    if (!ctx || !in || !out) return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_create: null argument");
+    CKR(check_order(in, sort_order, "spb_consolidate_plan_create"));
+    if (in->n >= (1ull << 31)) return spb_fail(SPB_ERR_TOO_LARGE, "%llu entries: one array holds fewer than 2^31 (the reference's own cap, algorithm.hpp:419)", (ull)in->n);
+    CK(cudaSetDevice(ctx->device));
+    spb_cons_plan *p = new spb_cons_plan();
+    p->ctx = ctx;
+    p->rank = in->rank;
+    p->shape[0] = in->shape[0]; p->shape[1] = in->shape[1];
+    p->so[0] = sort_order[0]; p->so[1] = in->rank > 1 ? sort_order[1] : 0;
+    p->n = in->n;
+    p->bits_lo = in->rank > 1 ? bits_for(in->shape[p->so[1]]) : 0;
+    p->key_bits = bits_for(in->shape[p->so[0]]) + p->bits_lo;
+    p->keys = nullptr; p->perm = nullptr;
+    u32 runs = 0;
+    if (in->n) {
+        // what spb_sorted_permutation does: a stable sort with the entry numbers as payload, nothing dropped or merged
+        Scratch ws(ctx);
+        double *iota;
+        u32 *cnt;
+        int rc = ws.get(&iota, in->n);
+        if (!rc) rc = ws.zeroed(&cnt, 1);
+        spb_coo *sorted = nullptr;
+        if (!rc) {
+            ++ctx->launches, k_iota_bits<<<grid_for(in->n, 256, 1u << 16), 256, 0, ctx->stream>>>(in->n, iota);
+            spb_coo tmp = *in;
+            tmp.val = iota;
+            tmp.owned = false;
+            rc = consolidate_core(ctx, &tmp, p->so, p->so, POLICY_KEEP_ALL, false, 0, &sorted, nullptr);
+        }
+        if (!rc && sorted->n != in->n)
+            rc = spb_fail(SPB_ERR_CUDA, "spb_consolidate_plan_create: lost entries (%llu of %llu)", (ull)sorted->n, (ull)in->n);
+        if (!rc && (ctx->pool.alloc((void **)&p->keys, in->n * sizeof(u64)) != cudaSuccess ||
+                    ctx->pool.alloc((void **)&p->perm, in->n * sizeof(u32)) != cudaSuccess))
+            rc = spb_fail(SPB_ERR_CUDA, "spb_consolidate_plan_create: out of device memory (%llu entries)", (ull)in->n);
+        if (!rc) {
+            ++ctx->launches, k_plan_pack<<<grid_for(in->n, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(
+                sorted->idx[p->so[0]], in->rank > 1 ? sorted->idx[p->so[1]] : nullptr, sorted->val, (u32)in->n, p->bits_lo,
+                p->keys, p->perm, cnt);
+            cudaError_t e = cudaGetLastError();
+            if (e == cudaSuccess) e = cudaMemcpyAsync(&runs, cnt, sizeof runs, cudaMemcpyDeviceToHost, ctx->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+            if (e != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "spb_consolidate_plan_create: %s", cudaGetErrorString(e));
+        }
+        spb_coo_free(ctx, sorted);
+        if (rc) {
+            spb_consolidate_plan_destroy(p);
+            return rc;
+        }
+    }
+    *out = p;
+    if (n_runs) *n_runs = runs;
+    return SPB_OK;
+}
+
+int spb_consolidate_plan_run(spb_cons_plan *plan, const double *val, int policy, int zero_nan, spb_coo **out,
+                             spb_consolidate_stats *stats) {
+    if (!plan || !out) return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_run: null argument");
+    if (plan->n && !val) return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_run: null value pointer");
+    if (policy < 0 || policy > 2) return spb_fail(SPB_ERR_ARG, "unknown duplicate policy %d", policy);
+    if ((uintptr_t)val & 7u) return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_run: value pointer is not 8-byte aligned");
+    spb_ctx *ctx = plan->ctx;
+    CK(cudaSetDevice(ctx->device));
+    if (stats) memset(stats, 0, sizeof *stats);
+    Scratch ws(ctx);
+    const double *dval = val;
+    if (plan->n) {
+        // device memory is read in place; host memory is staged as spb_coo_upload stages it
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, val) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
+        if (at.type == cudaMemoryTypeDevice && at.device != ctx->device)
+            return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_run: values on device %d, the plan's context is on device %d",
+                            at.device, ctx->device);
+        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) {
+            double *staged;
+            CKR(ws.get(&staged, plan->n));
+            const XferJob job = {staged, const_cast<double *>(val), (size_t)plan->n * sizeof(double)};
+            CKR(staged_copy(ctx, &job, 1, true));
+            dval = staged;
+        }
+    }
+    spb_coo *r = nullptr;
+    CKR(coo_new(ctx, plan->rank, plan->shape, plan->n, true, &r));
+    set_order(r, plan->so);
+    if (plan->n == 0) { *out = r; return SPB_OK; }  // algorithm.hpp:263,318
+    int rc = 0;
+    if (plan->rank == 2) {  // the reduce pass also emits the compressed row starts of its output
+        const u64 ext = plan->shape[plan->so[0]];
+        const u64 cap = (plan->n < ext ? plan->n : ext) + 1;
+        if (ctx->pool.alloc((void **)&r->row_start, cap * sizeof(u32)) != cudaSuccess ||
+            ctx->pool.alloc((void **)&r->row_id, cap * sizeof(i32)) != cudaSuccess)
+            rc = spb_fail(SPB_ERR_CUDA, "out of device memory");
+    }
+    if (!rc) rc = cons_plan_run(plan, dval, policy, zero_nan, r, stats);
+    if (rc) { spb_coo_free(ctx, r); return rc; }
+    *out = r;
+    return SPB_OK;
+}
+
+int spb_consolidate_plan_destroy(spb_cons_plan *plan) {
+    if (!plan) return SPB_OK;
+    plan->ctx->pool.release(plan->keys);
+    plan->ctx->pool.release(plan->perm);
+    delete plan;
+    return SPB_OK;
 }
 
 }  // extern "C"
