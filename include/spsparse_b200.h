@@ -222,6 +222,43 @@ int spb_mm_plan_symbolic(spb_mm_plan *plan, uint64_t panel, spb_mm_stats *stats)
 int spb_mm_plan_panel(spb_mm_plan *plan, uint64_t panel, spb_coo **out, spb_mm_stats *stats /* may be NULL */);
 int spb_mm_plan_destroy(spb_mm_plan *plan);
 
+/* ---- multiply with a fixed operand pattern ----------------------------------------------------------------------
+ * For callers that multiply operands of the same (row, column) patterns again and again with new values (a time step that
+ * assembles A and B every step): everything spb_multiply_mm does that depends only on the indices -- the consolidations'
+ * sorts, the row structure, the densified scale vectors and the whole symbolic phase -- is done once.
+ *
+ * spb_mm_pattern_create  fixes the index arrays of A and B with their sort flags, both transpose flags, C, policy, zero_nan and
+ *                        the three scale vectors (pattern and values: a zero scale masks rows and columns).  The values of A,
+ *                        B are not read.  The plan copies what it needs: A, B and the scale vectors may be freed afterwards.
+ *                        nnz_bound (may be NULL): outputs of the full pattern, a bound on every run's nnz.  A pattern whose
+ *                        product has 2^31 entries or more fails with SPB_ERR_TOO_LARGE (use row panels, spb_mm_plan_create).
+ *                        Device memory of the plan, from the context's pool: per raw entry of A or B 4 bytes (8 for B with
+ *                        zero_nan; 16 for an operand used as it is flagged); per run of equal indices 21 bytes, plus 8 per run
+ *                        of A; per non-empty row of op(A) 13 bytes; per product of a hash-bin row 4 bytes, per hash-bin row
+ *                        about 24 bytes per column window; the densified scale vectors (8 bytes per index, 9 for scalej) and
+ *                        B's dense pointer (4 bytes per inner index).
+ * spb_mm_pattern_run     what spb_multiply_mm(ctx, C, si, A', tA, sj, B', tB, sk, policy, zero_nan) returns, bit for bit, where
+ *                        A' / B' have the plan's indices and the values a_val (A.n doubles in A's entry order) / b_val (B.n in
+ *                        B's).  Device memory of the plan's device (any 8-byte alignment) or host memory (staged as
+ *                        spb_coo_upload stages it); a_val and b_val may be the same pointer.  When values empty a whole run of
+ *                        equal indices (zeros, or NaNs of the leading run with zero_nan) the run takes the full multiply on the
+ *                        remaining runs (stats->fallback); otherwise only the numeric kernels run.  Every row the register
+ *                        merge does not take goes to the hash bin (stats->mm.rows_esc is 0 on the fast path).
+ * spb_mm_pattern_destroy releases the plan; call it before destroying the plan's context. */
+typedef struct spb_mm_pattern spb_mm_pattern;
+typedef struct {
+    int fallback;                        /* 1: a run was empty, the multiply ran on the compacted operands */
+    uint64_t empty_runs_a, empty_runs_b; /* runs of equal indices the values emptied */
+    float ms_fold_a, ms_fold_b;          /* folding the values into one per run (B in its reference order: the gather) */
+    spb_mm_stats mm;                     /* the multiply; on the fast path ms_prepare = ms_symbolic = 0 */
+} spb_mm_pattern_stats;
+int spb_mm_pattern_create(spb_ctx *ctx, double C, const spb_coo *scalei, const spb_coo *A, char transpose_A,
+                          const spb_coo *scalej, const spb_coo *B, char transpose_B, const spb_coo *scalek,
+                          int policy, int zero_nan, spb_mm_pattern **out, uint64_t *nnz_bound /* may be NULL */);
+int spb_mm_pattern_run(spb_mm_pattern *plan, const double *a_val, const double *b_val, spb_coo **out,
+                       spb_mm_pattern_stats *stats /* may be NULL */);
+int spb_mm_pattern_destroy(spb_mm_pattern *plan);
+
 /* ---- row-partitioned multiply on the GPUs of one node ---------------------------------------
  * One process per GPU.  The A-row loop of spsparse::multiply carries no state between rows
  * (multiply_sparse.hpp:192-246): every rank holds a block of the rows of A (blocks that tile A's rows in rank

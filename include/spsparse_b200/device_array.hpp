@@ -180,6 +180,48 @@ public:
     }
 };
 
+// multiply() for fixed operand patterns (spb_mm_pattern_*): the indices of A and B, the transpose flags, C, the scale vectors,
+// the policy and zero_nan are fixed at construction; run(a_val, b_val) returns multiply() of A's and B's indices with those
+// values (A.size() / B.size() doubles in entry order, device or host memory), bit for bit, without sorting or a symbolic phase.
+// A, B and the scale vectors may be destroyed once the plan exists.  Move-only.
+class MultiplyPattern {
+    spb_mm_pattern *h_ = nullptr;
+    size_t nnz_bound_ = 0;
+
+public:
+    MultiplyPattern() {}
+    MultiplyPattern(double C, DeviceCooArray<1> const *scalei, DeviceCooArray<2> const &A, char transpose_A,
+                    DeviceCooArray<1> const *scalej, DeviceCooArray<2> const &B, char transpose_B,
+                    DeviceCooArray<1> const *scalek, DuplicatePolicy policy = DuplicatePolicy::ADD, bool zero_nan = false) {
+        uint64_t bound = 0;
+        check(spb_mm_pattern_create(default_context(), C, scalei ? scalei->handle() : nullptr, A.handle(), transpose_A,
+                                    scalej ? scalej->handle() : nullptr, B.handle(), transpose_B,
+                                    scalek ? scalek->handle() : nullptr, policy_code(policy), zero_nan ? 1 : 0, &h_, &bound));
+        nnz_bound_ = (size_t)bound;
+    }
+    MultiplyPattern(MultiplyPattern const &) = delete;
+    MultiplyPattern &operator=(MultiplyPattern const &) = delete;
+    MultiplyPattern(MultiplyPattern &&o) noexcept : h_(o.h_), nnz_bound_(o.nnz_bound_) { o.h_ = nullptr; o.nnz_bound_ = 0; }
+    MultiplyPattern &operator=(MultiplyPattern &&o) noexcept {
+        if (this != &o) { reset(); h_ = o.h_; nnz_bound_ = o.nnz_bound_; o.h_ = nullptr; o.nnz_bound_ = 0; }
+        return *this;
+    }
+    ~MultiplyPattern() { reset(); }
+    void reset() {
+        if (h_) spb_mm_pattern_destroy(h_);
+        h_ = nullptr;
+        nnz_bound_ = 0;
+    }
+    spb_mm_pattern *handle() const { return h_; }
+    size_t nnz_bound() const { return nnz_bound_; }   // outputs of the full pattern: no run returns more
+
+    DeviceCooArray<2> run(const double *a_val, const double *b_val) const {
+        spb_coo *r = nullptr;
+        check(spb_mm_pattern_run(h_, a_val, b_val, &r, nullptr));
+        return DeviceCooArray<2>(r);
+    }
+};
+
 // C * diag(scalei) * op(A) * diag(scalej) * op(B) * diag(scalek); absent scale vectors: nullptr.  Operands need not be
 // consolidated (the library does what the reference's Consolidate<> does); the result is consolidated row-major.
 inline DeviceCooArray<2> multiply(double C, DeviceCooArray<1> const *scalei, DeviceCooArray<2> const &A, char transpose_A,

@@ -37,6 +37,11 @@ class MMStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class MMPatternStats(C.Structure):
+    _fields_ = [("fallback", C.c_int), ("empty_runs_a", C.c_uint64), ("empty_runs_b", C.c_uint64),
+                ("ms_fold_a", C.c_float), ("ms_fold_b", C.c_float), ("mm", MMStats)]
+
+
 class RowpartStats(C.Structure):
     _fields_ = [("a", ConsolidateStats), ("b", ConsolidateStats), ("mm", MMStats),
                 ("rows_fetched", C.c_uint64), ("entries_fetched", C.c_uint64),
@@ -86,6 +91,10 @@ SIGNATURES = {
     "spb_mm_plan_symbolic": (C.c_int, [vp, C.c_uint64, C.POINTER(MMStats)]),
     "spb_mm_plan_panel": (C.c_int, [vp, C.c_uint64, C.POINTER(vp), C.POINTER(MMStats)]),
     "spb_mm_plan_destroy": (C.c_int, [vp]),
+    "spb_mm_pattern_create": (C.c_int, [vp, C.c_double, vp, vp, C.c_char, vp, vp, C.c_char, vp, C.c_int, C.c_int,
+                                        C.POINTER(vp), u64p]),
+    "spb_mm_pattern_run": (C.c_int, [vp, vp, vp, C.POINTER(vp), C.POINTER(MMPatternStats)]),
+    "spb_mm_pattern_destroy": (C.c_int, [vp]),
     "spb_rowpart_create": (C.c_int, [vp, C.c_int, C.c_int, u64p, C.c_uint64, C.POINTER(vp)]),
     "spb_rowpart_handle": (C.c_int, [vp, vp, C.c_uint64]),
     "spb_rowpart_attach": (C.c_int, [vp, vp, C.c_uint64]),

@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import ConsolidateStats, MMStats, check, vp
+from ._lib import ConsolidateStats, MMPatternStats, MMStats, check, vp
 
 LEAVE_ALONE, ADD, REPLACE = 0, 1, 2  # DuplicatePolicy, spsparse.hpp:25-26
 ROW_MAJOR, COL_MAJOR = (0, 1), (1, 0)  # spsparse.cpp:30-31
@@ -203,6 +203,24 @@ def consolidate(ctx: Context, A: CooArray, sort_order, duplicate_policy=ADD, zer
     return (out, st) if stats else out
 
 
+def _plan_values(values, n):
+    """(pointer, keep-alive) for n values given to a plan run: a CUDA float64 tensor, a numpy array (host memory) or a raw
+    device pointer."""
+    if isinstance(values, int):
+        return values, None
+    if isinstance(values, np.ndarray):
+        v = np.ascontiguousarray(values, dtype=np.float64)
+        if v.ndim != 1 or v.shape[0] != n:
+            raise ValueError(f"values: {v.shape} for a plan of {n} entries")
+        return v.ctypes.data, v
+    if hasattr(values, "data_ptr") and getattr(values, "is_cuda", False):
+        import torch
+        if values.dtype != torch.float64 or values.dim() != 1 or values.numel() != n or values.stride(0) != 1:
+            raise ValueError(f"values: need a contiguous float64 tensor of {n} entries")
+        return values.data_ptr(), values
+    raise TypeError("values: a CUDA float64 tensor, a numpy array or a device pointer")
+
+
 class ConsolidatePlan:
     """``consolidate`` for a fixed index pattern (spb_consolidate_plan_*): the pattern of ``A`` is sorted once, and every
     ``run(values)`` returns what ``consolidate`` returns for ``A``'s indices with those values -- bit for bit -- with one
@@ -217,20 +235,7 @@ class ConsolidatePlan:
         self.h, self.n_runs = h, int(runs.value)
 
     def _values(self, values):
-        """(pointer, keep-alive) for a CUDA float64 tensor, a numpy array (host memory) or a raw device pointer."""
-        if isinstance(values, int):
-            return values, None
-        if isinstance(values, np.ndarray):
-            v = np.ascontiguousarray(values, dtype=np.float64)
-            if v.ndim != 1 or v.shape[0] != self.n:
-                raise ValueError(f"values: {v.shape} for a plan of {self.n} entries")
-            return v.ctypes.data, v
-        if hasattr(values, "data_ptr") and getattr(values, "is_cuda", False):
-            import torch
-            if values.dtype != torch.float64 or values.dim() != 1 or values.numel() != self.n or values.stride(0) != 1:
-                raise ValueError(f"values: need a contiguous float64 tensor of {self.n} entries")
-            return values.data_ptr(), values
-        raise TypeError("values: a CUDA float64 tensor, a numpy array or a device pointer")
+        return _plan_values(values, self.n)
 
     def run(self, values, duplicate_policy=ADD, zero_nan=False, stats=False):
         ptr, _keep = self._values(values)   # _keep: a converted numpy copy must outlive the call
@@ -243,6 +248,40 @@ class ConsolidatePlan:
     def free(self):
         if self.h:
             self.ctx.lib.spb_consolidate_plan_destroy(self.h)
+            self.h = None
+
+
+class MultiplyPattern:
+    """``multiply`` for fixed operand patterns (spb_mm_pattern_*): the indices of ``A`` and ``B``, both transpose flags, ``Cst``,
+    the scale vectors, the policy and ``zero_nan`` are fixed once, and every ``run(a_values, b_values)`` returns what
+    ``multiply`` returns for ``A``'s and ``B``'s indices with those values -- bit for bit -- without sorting anything or
+    repeating the symbolic phase.  ``A``, ``B`` and the scale vectors may be freed once the pattern exists.  Values are
+    ``A.size()`` / ``B.size()`` doubles in entry order: CUDA float64 tensors, numpy arrays or device pointers (the same object
+    may be passed twice); device values are read on the context's stream."""
+
+    def __init__(self, ctx: Context, Cst, scalei, A, transpose_A, scalej, B, transpose_B, scalek,
+                 duplicate_policy=ADD, zero_nan=False):
+        self.ctx = ctx
+        self.n_a, self.n_b = A.size(), B.size()
+        h, bound = vp(), C.c_uint64()
+        check(ctx.lib.spb_mm_pattern_create(ctx.h, float(Cst), _h(scalei), A.h, transpose_A.encode(), _h(scalej), B.h,
+                                            transpose_B.encode(), _h(scalek), int(duplicate_policy), int(bool(zero_nan)),
+                                            C.byref(h), C.byref(bound)))
+        self.h, self.nnz_bound = h, int(bound.value)
+
+    def run(self, a_values, b_values, stats=False):
+        pa, _ka = _plan_values(a_values, self.n_a)   # _ka / _kb: converted numpy copies must outlive the call
+        pb, _kb = _plan_values(b_values, self.n_b)
+        if b_values is a_values:
+            pb = pa   # one array for both operands: one staging of host values
+        h, st = vp(), MMPatternStats()
+        check(self.ctx.lib.spb_mm_pattern_run(self.h, vp(pa) if pa else None, vp(pb) if pb else None, C.byref(h), C.byref(st)))
+        out = CooArray(self.ctx, h)
+        return (out, st) if stats else out
+
+    def free(self):
+        if self.h:
+            self.ctx.lib.spb_mm_pattern_destroy(self.h)
             self.h = None
 
 

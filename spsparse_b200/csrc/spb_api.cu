@@ -28,6 +28,7 @@
 #include "dense_ops.cuh"
 #include "rowpart.cuh"
 #include "cons_plan.cuh"
+#include "mm_pattern.cuh"
 
 thread_local std::string g_last_error;
 
@@ -1151,11 +1152,68 @@ struct PreScale {   // scalej already in dense form (the row-partitioned multipl
     const unsigned char *sj_mask;
 };
 
-static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_coo *A, int a_row_dim,
-                         const spb_coo *sj, const spb_coo *B, int b_inner_dim, const spb_coo *sk,
-                         spb_coo *out, spb_mm_stats *st, Timer &tm, int t_begin, bool symbolic_only = false,
-                         const PreScale *pre = nullptr) {
-    Scratch ws(ctx);
+// What the numeric half of a multiply reads: everything the symbolic half found, all of it depending only on the pattern of
+// the operands and the scale vectors (the register-merge count and the hash bin's bitmap pass read no values).  The device
+// arrays belong to the Scratch the symbolic half was given.
+struct MmState {
+    MMOperands m;
+    u64 nnz_a, nnz_b;
+    ull h_stats[8];           // as multiply_core's stats[] (see k_esc_row_products)
+    ull staged_blocks;
+    int nl_fit, nl_num, local_carve, blk_num;
+    bool local_count;
+    unsigned char *row_cls;
+    u32 *row_cnt;
+    u64 *c_ptr;
+    u64 nnz_c;                // counting outputs that will cancel to exactly 0
+    HashArgs ha;
+    u32 hash_cap;
+    u32 h_items;
+    bool items_ready;         // the hash bin's work items and window searches exist (mm_hash_items ran)
+    std::vector<EscChunk> chunks;
+    u32 *esc_first;
+    int t_prep, t_mcount, t_bins, t_hcount, t_esc, t_sym;   // marks of the symbolic half; t_prep < 0: it ran on another timer
+};
+
+// The hash bin's work items (k_hash_items) and, for rows cut into several items, where every item's window begins in every B
+// row (k_hash_splits): structure only, written into s.ha.
+static int mm_hash_items(spb_ctx *ctx, Scratch &ws, MmState &s, Timer &tm, int *t_emit, int *t_split) {
+    HashArgs &ha = s.ha;
+    const MMOperands &m = s.m;
+    const u32 cap = (u32)ctx->sm_count * 32;
+    const u64 max_items = s.h_stats[5] + s.nnz_c / s.hash_cap + 1;
+    CKR(ws.get(&ha.items, max_items));
+    CKR(ws.get(&ha.item_key, max_items));
+    ha.c_ptr = s.c_ptr;
+    ++ctx->launches, k_hash_items<<<grid_for((u64)ha.nrows * 32, 256, (u32)ctx->sm_count * 8), 256, 0, ctx->stream>>>(m, ha);
+    CK(cudaGetLastError());
+    ull h_split = 0;
+    *t_emit = *t_split = tm.mark();
+    CK(cudaMemcpyAsync(&s.h_items, ha.n_items, sizeof(u32), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h_split, ha.split_total, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (h_split) {
+        // rows cut into several items: where every item's column window begins in every B row of the row
+        u32 *split;
+        CKR(ws.get(&split, h_split));
+        ++ctx->launches, k_hash_splits<<<s.h_items < cap * 4 ? s.h_items : cap * 4, 256, 0, ctx->stream>>>(m, ha, s.h_items, split);
+        CK(cudaGetLastError());
+        ha.split = split;
+        *t_split = tm.mark();
+    }
+    s.items_ready = true;
+    return 0;
+}
+
+// Symbolic half: prepares the operands (row index of A, dense pointer of B, densified scale vectors), bins the rows and places
+// them.  *done: the call is complete without the numeric half (symbolic_only, or the one-pass merge went through and wrote
+// `out`).  pattern (spb_mm_pattern_create): every row the register merge does not take goes to the hash bin -- expand-sort-
+// compress forms values in its symbolic phase -- and the one-pass merge is never tried.
+static int mm_symbolic(spb_ctx *ctx, Scratch &ws, double C, const spb_coo *si, const spb_coo *A, int a_row_dim,
+                       const spb_coo *sj, const spb_coo *B, int b_inner_dim, const spb_coo *sk,
+                       spb_coo *out, spb_mm_stats *st, Timer &tm, int t_begin, bool symbolic_only,
+                       const PreScale *pre, bool pattern, MmState &s, bool *done) {
+    *done = false;
     const int a_in = 1 - a_row_dim, b_col = 1 - b_inner_dim;
     const u64 m_rows = A->shape[a_row_dim], n_inner = A->shape[a_in], n_cols = B->shape[b_col];
     MMOperands m;
@@ -1203,7 +1261,7 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
         const double avg_a_len = nrows ? (double)m.nnz_a / (double)nrows : 0.0;
         const double avg_b = n_inner ? (double)B->n / (double)n_inner : 0.0;
         const u64 cap_out = (u64)nrows * 16;
-        const bool want = !symbolic_only && nrows && avg_a_len * avg_b <= 40.0 && (A->max_row_len == 0 || A->max_row_len <= (u32)MERGE_MAX_LISTS) &&
+        const bool want = !symbolic_only && !pattern && nrows && avg_a_len * avg_b <= 40.0 && (A->max_row_len == 0 || A->max_row_len <= (u32)MERGE_MAX_LISTS) &&
                           cap_out < (1ull << 31) && cap_out * 16 <= (48ull << 30) &&
                           getenv("SPB_MERGE_ONEPASS") && atoi(getenv("SPB_MERGE_ONEPASS")) != 0;
         if (want) {
@@ -1259,6 +1317,7 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
                             st->ms_merge_numeric = st->ms_numeric;
                             st->ms_total = tm.ms(t_begin, t_one);
                         }
+                        *done = true;
                         return SPB_OK;
                     }
                     ctx->pool.release(ci); ctx->pool.release(ck); ctx->pool.release(cv);
@@ -1356,7 +1415,8 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
         ++ctx->launches, k_entry_products<<<grid_for(m.nnz_a, 256, cap), 256, 0, ctx->stream>>>(m, A->idx[a_row_dim], ent_f);
         CKR((exclusive_scan<u32, u64>(ctx, ws, ent_f, ent_off, m.nnz_a)));
         // second-level bin: long rows with enough products use the bitmap + hash accumulators (needs the columns to fit the bitmap)
-        const bool hash_ok = ctx->hash_min_products != ~0ull;
+        const u64 hash_min = pattern ? 0 : ctx->hash_min_products;
+        const bool hash_ok = hash_min != ~0ull;
         u32 *hash_rows_big = nullptr;
         if (hash_ok) { CKR(ws.get(&hash_rows, h_stats[2])); CKR(ws.get(&hash_rows_big, h_stats[2])); }
         // rows of at most HSM_CAP products: columns listed by a sort in shared memory (SPB_HASH_SMALL=0: everything by bitmap)
@@ -1366,7 +1426,7 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
         const char *hs_env = getenv("SPB_HASH_SMALL");
         const bool wide = n_cols > (getenv("SPB_HASH_WIN_COLS") ? strtoull(getenv("SPB_HASH_WIN_COLS"), nullptr, 10) : (u64)HASH_MAX_COLS);
         const u64 small_max = (hs_env ? atoi(hs_env) != 0 : wide) ? (u64)HSM_CAP : 0;
-        ++ctx->launches, k_esc_row_products<<<grid_for(nrows, 256, cap), 256, 0, ctx->stream>>>(m, ent_off, row_cls, esc_f, ctx->hash_min_products, small_max, hash_rows, hash_rows_big, stats);
+        ++ctx->launches, k_esc_row_products<<<grid_for(nrows, 256, cap), 256, 0, ctx->stream>>>(m, ent_off, row_cls, esc_f, hash_min, small_max, hash_rows, hash_rows_big, stats);
         CK(cudaGetLastError());
         ull h_long[8];
         CK(cudaMemcpyAsync(h_long, stats, sizeof h_long, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1521,8 +1581,38 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
             st->ms_hash_count = tm.ms(t_bins, t_hcount);
             st->ms_esc = tm.ms(t_hcount, t_esc);
         }
+        *done = true;
         return SPB_OK;
     }
+    s.m = m;
+    s.nnz_a = A->n; s.nnz_b = B->n;
+    memcpy(s.h_stats, h_stats, sizeof h_stats);
+    s.staged_blocks = staged_blocks;
+    s.nl_fit = nl_fit; s.nl_num = nl_num; s.local_carve = local_carve; s.blk_num = blk_num;
+    s.local_count = local_count;
+    s.row_cls = row_cls; s.row_cnt = row_cnt; s.c_ptr = c_ptr; s.nnz_c = nnz_c;
+    s.ha = ha; s.hash_cap = hash_cap;
+    s.h_items = 0; s.items_ready = false;
+    s.chunks = chunks; s.esc_first = esc_first;
+    s.t_prep = t_prep; s.t_mcount = t_mcount; s.t_bins = t_bins; s.t_hcount = t_hcount; s.t_esc = t_esc; s.t_sym = t_sym;
+    return SPB_OK;
+}
+
+// Numeric half: forms C on the placement the symbolic half made, reading the values s.m.a_val / s.m.b_val.
+static int mm_numeric(spb_ctx *ctx, Scratch &ws, MmState &s, spb_coo *out, spb_mm_stats *st, Timer &tm, int t_begin) {
+    const MMOperands &m = s.m;
+    const u32 nrows = m.nrows;
+    const ull *h_stats = s.h_stats;
+    u64 nnz_c = s.nnz_c;
+    u64 *c_ptr = s.c_ptr;
+    unsigned char *row_cls = s.row_cls;
+    HashArgs &ha = s.ha;
+    const u32 cap = (u32)ctx->sm_count * 32;
+    const int blk_num = s.blk_num, local_carve = s.local_carve, nl_num = s.nl_num, nl_fit = s.nl_fit;
+    const bool local_count = s.local_count;
+    const ull staged_blocks = s.staged_blocks;
+    const int t_sym = s.t_sym;
+    const double h0 = now_ms();
     if (nnz_c >= (1ull << 31))
         return spb_fail(SPB_ERR_TOO_LARGE, "product has %llu entries; a VectorCooArray holds < 2^31 (algorithm.hpp:419) -- "
                         "form it in row panels (spb_mm_plan_create)", (ull)nnz_c);
@@ -1566,34 +1656,20 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
 #undef SPB_LAUNCH_NUM
     }
     const int t_mnum = tm.mark();
-    for (auto &ch : chunks)
-        if (ch.n) ++ctx->launches, k_esc_copy<<<grid_for(ch.n, 256, cap), 256, 0, ctx->stream>>>(ch.row, ch.k, ch.v, ch.n, esc_first, c_ptr, m.arow_id, out->idx[0], out->idx[1], out->val);
+    for (auto &ch : s.chunks)
+        if (ch.n) ++ctx->launches, k_esc_copy<<<grid_for(ch.n, 256, cap), 256, 0, ctx->stream>>>(ch.row, ch.k, ch.v, ch.n, s.esc_first, c_ptr, m.arow_id, out->idx[0], out->idx[1], out->val);
     u32 h_shrunk = 0;
     int t_hemit0 = tm.mark(), t_hemit1 = t_hemit0, t_hsplit = t_hemit0, t_hnum = t_hemit0;
     if (h_stats[5] && nnz_c) {
         // the rows are placed: cut them into work items (the columns were listed by the bitmap pass of the symbolic phase)
-        u32 h_items = 0;
-        const u64 max_items = h_stats[5] + nnz_c / hash_cap + 1;
-        CKR(ws.get(&ha.items, max_items));
-        CKR(ws.get(&ha.item_key, max_items));
-        ha.c_ptr = c_ptr; ha.c_i = out->idx[0]; ha.c_k = out->idx[1]; ha.c_v = out->val;
-        ++ctx->launches, k_hash_items<<<grid_for((u64)ha.nrows * 32, 256, (u32)ctx->sm_count * 8), 256, 0, ctx->stream>>>(m, ha);
-        CK(cudaGetLastError());
-        ull h_split = 0;
-        t_hemit1 = t_hsplit = t_hnum = tm.mark();
-        CK(cudaMemcpyAsync(&h_items, ha.n_items, sizeof(u32), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaMemcpyAsync(&h_split, ha.split_total, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        if (h_split) {
-            // rows cut into several items: where every item's column window begins in every B row of the row
-            u32 *split;
-            CKR(ws.get(&split, h_split));
-            ++ctx->launches, k_hash_splits<<<h_items < cap * 4 ? h_items : cap * 4, 256, 0, ctx->stream>>>(m, ha, h_items, split);
-            CK(cudaGetLastError());
-            ha.split = split;
-            t_hsplit = t_hnum = tm.mark();
+        if (!s.items_ready) {
+            CKR(mm_hash_items(ctx, ws, s, tm, &t_hemit1, &t_hsplit));
+            t_hnum = t_hsplit;
         }
+        ha.c_i = out->idx[0]; ha.c_k = out->idx[1]; ha.c_v = out->val;
+        const u32 h_items = s.h_items;
         if (h_items) {
+            ha.dbg = nullptr;
             if (tracing()) CKR(ws.zeroed(&ha.dbg, 16));
             ++ctx->launches;
             if (ctx->hash_variant == 2) {
@@ -1652,20 +1728,34 @@ static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_co
     if (st) {
         st->products = h_stats[0] + h_stats[3] + h_stats[4]; st->rows_merge = h_stats[1]; st->rows_esc = h_stats[2] - h_stats[5];
         st->products_esc = h_stats[3]; st->rows_hash = h_stats[5]; st->products_hash = h_stats[4];
-        st->nnz_a = A->n; st->nnz_b = B->n; st->rows_a = nrows; st->nnz_c = nnz_c;
-        st->ms_prepare = tm.ms(t_begin, t_prep);
-        st->ms_symbolic = tm.ms(t_prep, t_sym);
+        st->nnz_a = s.nnz_a; st->nnz_b = s.nnz_b; st->rows_a = nrows; st->nnz_c = nnz_c;
+        if (s.t_prep >= 0) {
+            st->ms_prepare = tm.ms(t_begin, s.t_prep);
+            st->ms_symbolic = tm.ms(s.t_prep, t_sym);
+            st->ms_merge_count = tm.ms(s.t_prep, s.t_mcount);
+            st->ms_hash_count = tm.ms(s.t_bins, s.t_hcount);
+            st->ms_esc = tm.ms(s.t_hcount, s.t_esc);
+        }
         st->ms_numeric = tm.ms(t_sym, t_num);
         st->ms_total = tm.ms(t_begin, t_num);
-        st->ms_merge_count = tm.ms(t_prep, t_mcount);
-        st->ms_hash_count = tm.ms(t_bins, t_hcount);
-        st->ms_esc = tm.ms(t_hcount, t_esc);
         st->ms_merge_numeric = tm.ms(t_sym, t_mnum);
         st->ms_hash_emit = tm.ms(t_hemit0, t_hemit1);
         st->ms_hash_splits = tm.ms(t_hemit1, t_hsplit);
         st->ms_hash_numeric = tm.ms(t_hsplit, t_hnum);
     }
     return SPB_OK;
+}
+
+static int multiply_core(spb_ctx *ctx, double C, const spb_coo *si, const spb_coo *A, int a_row_dim,
+                         const spb_coo *sj, const spb_coo *B, int b_inner_dim, const spb_coo *sk,
+                         spb_coo *out, spb_mm_stats *st, Timer &tm, int t_begin, bool symbolic_only = false,
+                         const PreScale *pre = nullptr) {
+    Scratch ws(ctx);
+    MmState s;
+    bool done = false;
+    CKR(mm_symbolic(ctx, ws, C, si, A, a_row_dim, sj, B, b_inner_dim, sk, out, st, tm, t_begin, symbolic_only, pre, false, s, &done));
+    if (done) return SPB_OK;
+    return mm_numeric(ctx, ws, s, out, st, tm, t_begin);
 }
 
 // ==================================================================================================
@@ -2057,6 +2147,23 @@ struct spb_cons_plan {
     u32 *perm;   // [n] sorted position -> entry number
 };
 
+// n values given to a plan run: device memory is read in place; host memory is staged as spb_coo_upload stages it
+static int device_values(spb_ctx *ctx, Scratch &ws, const double *val, u64 n, const char *what, const double **dval) {
+    *dval = val;
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, val) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
+    if (at.type == cudaMemoryTypeDevice && at.device != ctx->device)
+        return spb_fail(SPB_ERR_ARG, "%s: values on device %d, the plan's context is on device %d", what, at.device, ctx->device);
+    if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) {
+        double *staged;
+        CKR(ws.get(&staged, n));
+        const XferJob job = {staged, const_cast<double *>(val), (size_t)n * sizeof(double)};
+        CKR(staged_copy(ctx, &job, 1, true));
+        *dval = staged;
+    }
+    return 0;
+}
+
 // the reduce of the kept pairs into r (allocated for plan->n entries); statistics as spb_consolidate_stats describes
 static int cons_plan_run(spb_cons_plan *plan, const double *dval, int policy, int zero_nan, spb_coo *r,
                          spb_consolidate_stats *st) {
@@ -2194,21 +2301,7 @@ int spb_consolidate_plan_run(spb_cons_plan *plan, const double *val, int policy,
     if (stats) memset(stats, 0, sizeof *stats);
     Scratch ws(ctx);
     const double *dval = val;
-    if (plan->n) {
-        // device memory is read in place; host memory is staged as spb_coo_upload stages it
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, val) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
-        if (at.type == cudaMemoryTypeDevice && at.device != ctx->device)
-            return spb_fail(SPB_ERR_ARG, "spb_consolidate_plan_run: values on device %d, the plan's context is on device %d",
-                            at.device, ctx->device);
-        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) {
-            double *staged;
-            CKR(ws.get(&staged, plan->n));
-            const XferJob job = {staged, const_cast<double *>(val), (size_t)plan->n * sizeof(double)};
-            CKR(staged_copy(ctx, &job, 1, true));
-            dval = staged;
-        }
-    }
+    if (plan->n) CKR(device_values(ctx, ws, val, plan->n, "spb_consolidate_plan_run", &dval));
     spb_coo *r = nullptr;
     CKR(coo_new(ctx, plan->rank, plan->shape, plan->n, true, &r));
     set_order(r, plan->so);
@@ -2232,6 +2325,319 @@ int spb_consolidate_plan_destroy(spb_cons_plan *plan) {
     plan->ctx->pool.release(plan->keys);
     plan->ctx->pool.release(plan->perm);
     delete plan;
+    return SPB_OK;
+}
+
+}  // extern "C"
+
+// ---- multiply with a fixed operand pattern -----------------------------------------------------------------------------
+// Everything spb_multiply_mm does that depends only on the operands' indices and the scale vectors -- the consolidations'
+// sorts, the row index of A, B's dense pointer, the densified scale vectors, the whole symbolic phase -- is done once at
+// creation.  A run folds the new values into one slot per run of equal indices (mm_pattern.cuh) and, when no run came out
+// empty, runs only the numeric kernels on the placement the creation made.  When a run is empty the operands' patterns are
+// smaller than the plan's: the non-empty runs are compacted -- exactly what spb_multiply_mm's consolidations return -- and the
+// whole multiply runs on them.
+enum { PO_FOLD = 0, PO_GATHER = 1, PO_AS_GIVEN = 2 };
+struct PatternOperand {
+    int mode;                       // PO_FOLD: consolidated by spb_multiply_mm; PO_GATHER: B flagged in the reference's order
+                                    // (re-bucketed, every entry kept); PO_AS_GIVEN: A flagged (row, inner), used as it is
+    u32 n = 0, runs = 0;            // entries of the value array; entries of `full`
+    u32 *perm = nullptr;            // [n] sorted position -> entry number (PO_FOLD, PO_GATHER)
+    u32 *off = nullptr;             // [runs + 1] first sorted position of every run (PO_FOLD)
+    u32 *ref_pos = nullptr;         // [n] B with zero_nan: sorted entry -> position in the reference's order (PO_FOLD)
+    unsigned char *live = nullptr;  // [runs] set by a fold (PO_FOLD)
+    spb_coo *full = nullptr;        // the operand with every run present, one entry per run; full->val holds the folded values
+};
+
+struct spb_mm_pattern {
+    spb_ctx *ctx;
+    double C;
+    int policy, zero_nan;
+    u64 shape[2];
+    bool empty;                     // the product is empty whatever the values (C = 0, an empty scale vector or operand)
+    int a_row_dim, b_inner_dim;
+    spb_coo *si = nullptr, *sj = nullptr, *sk = nullptr;   // copies of the scale vectors
+    PatternOperand A, B;
+    Scratch *sym = nullptr;         // device memory of the symbolic phase
+    MmState s;
+};
+
+// Sorts `in` by `so` once (stable, every entry kept, the entry numbers as payload).  PO_FOLD: the run offsets and the
+// consolidated index vectors of the full pattern, and with ref_so the reference positions; PO_GATHER: the sorted array itself.
+static int pattern_operand(spb_ctx *ctx, const spb_coo *in, const int *so, const int *ref_so, PatternOperand &op) {
+    const u32 n = (u32)in->n;
+    const u32 grid = (u32)ctx->sm_count * 16;
+    op.n = n;
+    Scratch ws(ctx);
+    double *iota;
+    CKR(ws.get(&iota, n));
+    ++ctx->launches, k_iota_bits<<<grid_for(n, 256, 1u << 16), 256, 0, ctx->stream>>>(n, iota);
+    spb_coo tmp = *in;
+    tmp.val = iota;
+    tmp.owned = false;
+    spb_coo *sorted = nullptr;
+    CKR(consolidate_core(ctx, &tmp, so, so, POLICY_KEEP_ALL, false, 0, &sorted, nullptr));
+    if (sorted->n != n) {
+        spb_coo_free(ctx, sorted);
+        return spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: lost entries (%llu of %u)", (ull)sorted->n, n);
+    }
+    const i32 *hi = sorted->idx[so[0]], *lo = sorted->idx[so[1]];
+    unsigned char *head;
+    CKR(ws.get(&head, n));
+    CK(ctx->pool.alloc((void **)&op.perm, (u64)n * sizeof(u32)));
+    ++ctx->launches, k_pattern_heads<<<grid_for(n, 256, grid), 256, 0, ctx->stream>>>(hi, lo, sorted->val, n, op.perm, head);
+    if (op.mode == PO_GATHER) {
+        op.runs = n;
+        op.full = sorted;   // its values (the entry numbers) are overwritten by every run
+        return 0;
+    }
+    u64 *slot;
+    CKR(ws.get(&slot, (u64)n + 1));
+    CKR((exclusive_scan<unsigned char, u64>(ctx, ws, head, slot, n)));
+    u64 runs = 0;
+    CK(cudaMemcpyAsync(&runs, slot + n, sizeof runs, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    op.runs = (u32)runs;
+    int rc = coo_new(ctx, 2, in->shape, runs, true, &op.full);
+    if (!rc) {
+        set_order(op.full, so);
+        if (ctx->pool.alloc((void **)&op.off, (runs + 1) * sizeof(u32)) != cudaSuccess ||
+            ctx->pool.alloc((void **)&op.live, runs) != cudaSuccess)
+            rc = spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: out of device memory (%llu runs)", (ull)runs);
+    }
+    if (!rc) {
+        ++ctx->launches, k_pattern_runs<<<grid_for(n, 256, grid), 256, 0, ctx->stream>>>(hi, lo, head, slot, n, op.off,
+                                                                                         op.full->idx[so[0]], op.full->idx[so[1]]);
+        if (cudaGetLastError() != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: launch failed");
+    }
+    spb_coo_free(ctx, sorted);
+    if (rc || !ref_so) return rc;
+    // the reference's order: sorted the same way; inv[entry] = its position there
+    spb_coo *ref = nullptr;
+    CKR(consolidate_core(ctx, &tmp, ref_so, ref_so, POLICY_KEEP_ALL, false, 0, &ref, nullptr));
+    u32 *inv;
+    rc = ws.get(&inv, n);
+    if (!rc && ctx->pool.alloc((void **)&op.ref_pos, (u64)n * sizeof(u32)) != cudaSuccess)
+        rc = spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: out of device memory (%u entries)", n);
+    if (!rc) {
+        ++ctx->launches, k_pattern_invert<<<grid_for(n, 256, grid), 256, 0, ctx->stream>>>(ref->val, n, inv);
+        ++ctx->launches, k_pattern_ref_pos<<<grid_for(n, 256, grid), 256, 0, ctx->stream>>>(op.perm, inv, n, op.ref_pos);
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(ctx->stream));   // inv dies with ws
+    }
+    spb_coo_free(ctx, ref);
+    return rc;
+}
+
+static void pattern_operand_free(spb_ctx *ctx, PatternOperand &op) {
+    ctx->pool.release(op.perm); ctx->pool.release(op.off); ctx->pool.release(op.ref_pos); ctx->pool.release(op.live);
+    spb_coo_free(ctx, op.full);
+    op.perm = op.off = op.ref_pos = nullptr; op.live = nullptr; op.full = nullptr;
+}
+
+// A run's values for one operand: folded into op.full->val (PO_FOLD; counters[0] += runs left empty, counters[1]: long runs),
+// gathered into it (PO_GATHER), or nothing to do (PO_AS_GIVEN).
+static int pattern_fold(spb_ctx *ctx, Scratch &ws, PatternOperand &op, const double *val, int policy, int zero_nan, u32 *counters) {
+    if (op.mode == PO_AS_GIVEN) return 0;
+    if (op.mode == PO_GATHER) {
+        ++ctx->launches, k_pattern_gather<<<grid_for(op.n, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(op.perm, val, op.n, op.full->val);
+        CK(cudaGetLastError());
+        return 0;
+    }
+    PatternFold f;
+    f.perm = op.perm; f.off = op.off; f.ref_pos = op.ref_pos; f.val = val; f.bound = nullptr;
+    f.runs = op.runs; f.policy = policy; f.out = op.full->val; f.live = op.live;
+    f.empty = counters; f.long_count = counters + 1;
+    f.long_cap = op.n / PF_LONG_RUN + 1;
+    CKR(ws.get(&f.long_list, f.long_cap));
+    if (zero_nan) {
+        u32 *bound;
+        CKR(ws.get(&bound, 1));
+        CK(cudaMemsetAsync(bound, 0xFF, sizeof(u32), ctx->stream));
+        if (op.ref_pos) {
+            ++ctx->launches, k_pattern_ref_bound<<<grid_for(op.n, 256, (u32)ctx->sm_count * 8), 256, 0, ctx->stream>>>(op.perm, op.ref_pos, val, op.n, bound);
+        } else {   // the reference sorts as the plan does: the first kept sorted position, found from the front
+            u32 *ticket;
+            CKR(ws.zeroed(&ticket, 1));
+            const u32 tiles = (u32)div_up(op.n, CP_TILE);
+            const u32 grid = tiles < (u32)ctx->sm_count * 2 ? tiles : (u32)ctx->sm_count * 2;
+            ++ctx->launches, k_plan_first_kept<<<grid, CP_THREADS, 0, ctx->stream>>>(op.perm, val, op.n, ticket, bound);
+        }
+        f.bound = bound;
+    }
+    ++ctx->launches, k_pattern_fold<<<grid_for(op.runs, 256, (u32)ctx->sm_count * 16), 256, 0, ctx->stream>>>(f);
+    ++ctx->launches, k_pattern_fold_long<<<(u32)ctx->sm_count * 4, 256, 0, ctx->stream>>>(f);
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// The non-empty runs of a folded operand, compacted: what spb_multiply_mm's consolidation returns for these values.
+static int pattern_compact(spb_ctx *ctx, Scratch &ws, const PatternOperand &op, u64 kept, spb_coo **out) {
+    spb_coo *r = nullptr;
+    CKR(coo_new(ctx, 2, op.full->shape, kept, true, &r));
+    set_order(r, op.full->sort_order);
+    u64 *slot;
+    int rc = ws.get(&slot, (u64)op.runs + 1);
+    if (!rc) rc = exclusive_scan<unsigned char, u64>(ctx, ws, op.live, slot, op.runs);
+    if (!rc) {
+        ++ctx->launches, k_compact_entries<<<grid_for(op.runs, 256, (u32)ctx->sm_count * 32), 256, 0, ctx->stream>>>(
+            op.runs, op.live, slot, op.full->idx[0], op.full->idx[1], op.full->val, r->idx[0], r->idx[1], r->val);
+        if (cudaGetLastError() != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "pattern compaction: launch failed");
+    }
+    if (rc) { spb_coo_free(ctx, r); return rc; }
+    *out = r;
+    return 0;
+}
+
+extern "C" {
+
+int spb_mm_pattern_destroy(spb_mm_pattern *plan) {
+    if (!plan) return SPB_OK;
+    spb_ctx *ctx = plan->ctx;
+    delete plan->sym;
+    pattern_operand_free(ctx, plan->A);
+    pattern_operand_free(ctx, plan->B);
+    spb_coo_free(ctx, plan->si); spb_coo_free(ctx, plan->sj); spb_coo_free(ctx, plan->sk);
+    delete plan;
+    return SPB_OK;
+}
+
+int spb_mm_pattern_create(spb_ctx *ctx, double C, const spb_coo *si, const spb_coo *A, char tA, const spb_coo *sj,
+                          const spb_coo *B, char tB, const spb_coo *sk, int policy, int zero_nan, spb_mm_pattern **out,
+                          uint64_t *nnz_bound) {
+    if (!ctx || !A || !B || !out) return spb_fail(SPB_ERR_ARG, "spb_mm_pattern_create: null argument");
+    if (A->rank != 2 || B->rank != 2) return spb_fail(SPB_ERR_ARG, "A and B must be rank-2 arrays");
+    if (policy < 0 || policy > 2) return spb_fail(SPB_ERR_ARG, "unknown duplicate policy %d", policy);
+    CKR(scale_ok(si, "scalei")); CKR(scale_ok(sj, "scalej")); CKR(scale_ok(sk, "scalek"));
+    if ((A->n && (!A->idx[0] || !A->idx[1])) || (B->n && (!B->idx[0] || !B->idx[1])))
+        return spb_fail(SPB_ERR_ARG, "spb_mm_pattern_create: A and B must be full COO arrays");
+    if (A->n >= (1ull << 31) || B->n >= (1ull << 31))
+        return spb_fail(SPB_ERR_TOO_LARGE, "one array holds fewer than 2^31 entries (the reference's own cap, algorithm.hpp:419)");
+    CK(cudaSetDevice(ctx->device));
+    const int a_so[2] = {tA == 'T' ? 1 : 0, tA == 'T' ? 0 : 1};
+    const int b_so[2] = {tB == 'T' ? 0 : 1, tB == 'T' ? 1 : 0};   // the reference's order: (col, inner)
+    const int b_mine[2] = {b_so[1], b_so[0]};                       // ours: (inner, col)
+    if (A->shape[a_so[1]] != B->shape[b_so[1]])
+        return spb_fail(SPB_ERR_INNER_DIM, "Inner dimensions for A (%ld) and B (%ld) must match!",
+                        (long)A->shape[a_so[1]], (long)B->shape[b_so[1]]);
+    spb_mm_pattern *p = new spb_mm_pattern();
+    p->ctx = ctx; p->C = C; p->policy = policy; p->zero_nan = zero_nan ? 1 : 0;
+    p->shape[0] = A->shape[a_so[0]]; p->shape[1] = B->shape[b_so[0]];
+    p->a_row_dim = a_so[0]; p->b_inner_dim = b_mine[0];
+    p->A.mode = (A->sort_order[0] == a_so[0] && A->sort_order[1] == a_so[1]) ? PO_AS_GIVEN : PO_FOLD;
+    p->B.mode = (B->sort_order[0] == b_so[0] && B->sort_order[1] == b_so[1]) ? PO_GATHER : PO_FOLD;
+    p->A.n = (u32)A->n; p->B.n = (u32)B->n;
+    p->empty = C == 0.0 || (si && si->n == 0) || A->n == 0 || (sj && sj->n == 0) || B->n == 0 || (sk && sk->n == 0);
+    int rc = 0;
+    if (!p->empty) {
+        if (si) rc = spb_coo_copy(ctx, si, &p->si);
+        if (!rc && sj) rc = spb_coo_copy(ctx, sj, &p->sj);
+        if (!rc && sk) rc = spb_coo_copy(ctx, sk, &p->sk);
+        if (!rc && p->A.mode == PO_AS_GIVEN) {
+            rc = coo_new(ctx, 2, A->shape, A->n, true, &p->A.full);
+            if (!rc) {
+                set_order(p->A.full, a_so);
+                p->A.runs = (u32)A->n;
+                for (int k = 0; k < 2 && !rc; ++k)
+                    if (cudaMemcpyAsync(p->A.full->idx[k], A->idx[k], A->n * sizeof(i32), cudaMemcpyDeviceToDevice, ctx->stream) != cudaSuccess)
+                        rc = spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: copy of A's indices failed");
+            }
+        } else if (!rc) {
+            rc = pattern_operand(ctx, A, a_so, nullptr, p->A);
+        }
+        if (!rc) rc = pattern_operand(ctx, B, b_mine, (p->B.mode == PO_FOLD && zero_nan) ? b_so : nullptr, p->B);
+        if (!rc) {
+            p->sym = new Scratch(ctx);
+            Timer tm(ctx->stream);
+            const int t0 = tm.mark();
+            bool done = false;
+            rc = mm_symbolic(ctx, *p->sym, C, p->si, p->A.full, p->a_row_dim, p->sj, p->B.full, p->b_inner_dim, p->sk, nullptr,
+                             nullptr, tm, t0, false, nullptr, true, p->s, &done);
+            if (!rc && p->s.nnz_c >= (1ull << 31))
+                rc = spb_fail(SPB_ERR_TOO_LARGE, "the pattern's product has %llu entries; a VectorCooArray holds < 2^31 (algorithm.hpp:419) -- "
+                              "form it in row panels (spb_mm_plan_create)", (ull)p->s.nnz_c);
+            int te, tsp;
+            if (!rc && p->s.h_stats[5] && p->s.nnz_c) rc = mm_hash_items(ctx, *p->sym, p->s, tm, &te, &tsp);
+            if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess)
+                rc = spb_fail(SPB_ERR_CUDA, "spb_mm_pattern_create: %s", cudaGetErrorString(cudaGetLastError()));
+            p->s.t_prep = -1;
+        }
+    }
+    if (rc) { spb_mm_pattern_destroy(p); return rc; }
+    *out = p;
+    if (nnz_bound) *nnz_bound = p->empty ? 0 : p->s.nnz_c;
+    return SPB_OK;
+}
+
+int spb_mm_pattern_run(spb_mm_pattern *plan, const double *a_val, const double *b_val, spb_coo **out,
+                       spb_mm_pattern_stats *stats) {
+    if (!plan || !out) return spb_fail(SPB_ERR_ARG, "spb_mm_pattern_run: null argument");
+    if ((plan->A.n && !a_val) || (plan->B.n && !b_val)) return spb_fail(SPB_ERR_ARG, "spb_mm_pattern_run: null value pointer");
+    if (((uintptr_t)a_val | (uintptr_t)b_val) & 7u) return spb_fail(SPB_ERR_ARG, "spb_mm_pattern_run: value pointer is not 8-byte aligned");
+    spb_ctx *ctx = plan->ctx;
+    CK(cudaSetDevice(ctx->device));
+    if (stats) memset(stats, 0, sizeof *stats);
+    spb_coo *r = nullptr;
+    CKR(coo_new(ctx, 2, plan->shape, 0, false, &r));
+    r->owned = true;
+    if (plan->empty) { *out = r; return SPB_OK; }
+    Scratch ws(ctx);
+    const double *da = a_val, *db = b_val;
+    int rc = device_values(ctx, ws, a_val, plan->A.n, "spb_mm_pattern_run", &da);
+    if (!rc) {
+        if (b_val == a_val) db = da;   // one array for both operands (A * diag(s) * A^T)
+        else rc = device_values(ctx, ws, b_val, plan->B.n, "spb_mm_pattern_run", &db);
+    }
+    Timer tm(ctx->stream);
+    const int t0 = tm.mark();
+    u32 *counters = nullptr;   // [0] A: runs left empty, [1] A: long runs, [2..3] the same for B
+    if (!rc) rc = ws.zeroed(&counters, 4);
+    if (!rc) rc = pattern_fold(ctx, ws, plan->A, da, plan->policy, plan->zero_nan, counters);
+    const int t1 = tm.mark();
+    if (!rc) rc = pattern_fold(ctx, ws, plan->B, db, plan->policy, plan->zero_nan, counters + 2);
+    const int t2 = tm.mark();
+    u32 h[4] = {0, 0, 0, 0};
+    if (!rc && cudaMemcpyAsync(h, counters, sizeof h, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "counter read-back failed");
+    if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "%s", cudaGetErrorString(cudaGetLastError()));
+    if (!rc && stats) {
+        stats->fallback = (h[0] || h[2]) ? 1 : 0;
+        stats->empty_runs_a = h[0]; stats->empty_runs_b = h[2];
+        stats->ms_fold_a = tm.ms(t0, t1); stats->ms_fold_b = tm.ms(t1, t2);
+    }
+    spb_mm_stats *mst = stats ? &stats->mm : nullptr;
+    if (!rc && !h[0] && !h[2]) {
+        // fast path: every run present, the operands have the plan's pattern -- only the numeric kernels run
+        MmState s = plan->s;
+        s.m.a_val = plan->A.mode == PO_AS_GIVEN ? da : plan->A.full->val;
+        s.m.b_val = plan->B.full->val;
+        if (s.ha.shrunk && cudaMemsetAsync(s.ha.shrunk, 0, sizeof(u32), ctx->stream) != cudaSuccess) rc = spb_fail(SPB_ERR_CUDA, "memset failed");
+        s.t_sym = tm.mark();
+        if (!rc) rc = mm_numeric(ctx, ws, s, r, mst, tm, s.t_sym);
+    } else if (!rc) {
+        // fallback: the operands spb_multiply_mm's consolidations return -- the non-empty runs -- through the whole multiply
+        spb_coo *Ac = nullptr, *Bc = nullptr;
+        spb_coo Aview;
+        const spb_coo *Ause = plan->A.full, *Buse = plan->B.full;
+        if (plan->A.mode == PO_AS_GIVEN) {
+            Aview = *plan->A.full;   // shares the plan's copy of the indices and its cached row structure
+            Aview.val = const_cast<double *>(da);
+            Aview.owned = false;
+            Ause = &Aview;
+        } else if (h[0]) {
+            rc = pattern_compact(ctx, ws, plan->A, plan->A.runs - h[0], &Ac);
+            Ause = Ac;
+        }
+        if (!rc && h[2]) {
+            rc = pattern_compact(ctx, ws, plan->B, plan->B.runs - h[2], &Bc);
+            Buse = Bc;
+        }
+        if (!rc && Ause->n && Buse->n)
+            rc = multiply_core(ctx, plan->C, plan->si, Ause, plan->a_row_dim, plan->sj, Buse, plan->b_inner_dim, plan->sk, r, mst, tm, t2);
+        spb_coo_free(ctx, Ac);
+        spb_coo_free(ctx, Bc);
+    }
+    if (rc) { spb_coo_free(ctx, r); return rc; }
+    *out = r;
     return SPB_OK;
 }
 
